@@ -25,6 +25,13 @@ Default (`--workload suite`) prints ONE JSON line (rank 0):
 port of the reference path alone (all cores, fork pool over batch rows) -- the reference is pure Python and cannot
 travel to the GPU box, so the port (oracle/py_oracle.py, pinned to fixtures generated from the unmodified reference)
 stands in for it.
+
+`--dump-outputs DIR` (the suite's headline and config1..config3) writes what the last timed step handed its caller,
+so that two builds can be compared output for output on identical seeded inputs (rank 0's batch at N > 1):
+  DIR/fgram_id.npy    float64 [B, L]
+  DIR/match_len.npy   float32 [B, L]
+  DIR/embeddings.npy  float32 [S, D]: the bf16 embeddings at S token positions (flat index b * L + l) drawn without
+                      replacement by numpy.random.default_rng(0) and sorted, S = min(B * L, 32 MiB / (4 * D))
 """
 
 from __future__ import annotations
@@ -253,8 +260,33 @@ def _fill_cache(cache, N, D, seed=2, std=0.02, chunk_bytes=1 << 30):
         cache.cache_embeddings(range(s, s + k), rows, verbose=False)
 
 
-def run_ours(args, w, rank, local_rank, world, name, steps=None):
-    """Returns the JSON line (a dict) on rank 0, None elsewhere.  Leaves the process group alive."""
+DUMP_EMBED_BYTES = 32 << 20     # float32 embeddings sample; the whole dump of config1..config3 stays under 64 MB
+
+
+def _snapshot_outputs(out, out_id, out_len):
+    """Device copies of a lookup's results, taken before the buffers are reused: fgram_id and match_len whole, the
+    embeddings at the fixed, seeded sample of positions described in the module docstring."""
+    import numpy as np
+    import torch
+    T, D = out_id.numel(), out.shape[-1]
+    n = min(T, DUMP_EMBED_BYTES // (4 * D))
+    pos = np.sort(np.random.default_rng(0).choice(T, size=n, replace=False))
+    return {"embeddings": out.view(T, D)[torch.from_numpy(pos).to(out.device)],
+            "fgram_id": out_id.clone(), "match_len": out_len.clone()}
+
+
+def _dump_outputs(snap, out_dir):
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in snap.items():
+        a = t.cpu().to(torch.float64 if name == "fgram_id" else torch.float32)    # exact: bf16, int32 and uint8 values
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
+def run_ours(args, w, rank, local_rank, world, name, dump_dir=None):
+    """Returns the JSON line (a dict) on rank 0, None elsewhere.  Leaves the process group alive.  With `dump_dir`, rank 0
+    writes the results of the last timed step there (see the module docstring)."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -284,7 +316,7 @@ def run_ours(args, w, rank, local_rank, world, name, steps=None):
 
     B, L, D, N, V = w["B"], w["L"], w["D"], w["N"], w["V"]
     T = B * L
-    steps = steps or args.steps
+    steps = args.steps
     # ---- build (untimed): the drop-in objects -- extractor (vocabulary + device index), cache (table), fallback rows ----
     toks, lens, longest = S.make_vocab_device(N, w["max_n"], V, seed=0, device=dev, return_longest=True)
     ex = sb.NGramExtractor.from_arrays(toks.cpu().numpy(), lens.cpu().numpy(), device=dev)
@@ -353,6 +385,8 @@ def run_ours(args, w, rank, local_rank, world, name, steps=None):
             stream.synchronize()
             barrier()
             ms = e0.elapsed_time(e1)
+            # the results of the timed replay's last step; the replays and e2e steps below overwrite the buffers
+            snap = _snapshot_outputs(out, out_id, out_len) if dump_dir else None
             repeats = []
             for _ in range(4):                       # variance only; `value` is the ONE timed replay above
                 r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -389,7 +423,6 @@ def run_ours(args, w, rank, local_rank, world, name, steps=None):
     h_id = torch.empty((B, L), dtype=torch.int32).pin_memory()
     h_len = torch.empty((B, L), dtype=torch.uint8).pin_memory()
     d_ids = torch.empty((B, L), dtype=torch.int64, device=dev)
-    e2e_steps = steps if T * D * 2 < (1 << 30) else max(3, min(steps, 8))
 
     def e2e_step(k, h_emb=None):
         d_ids.copy_(h_ids[k % N_BATCHES], non_blocking=True)
@@ -436,13 +469,13 @@ def run_ours(args, w, rank, local_rank, world, name, steps=None):
 
     pipe_value = time_pipelined()
     h_emb = torch.empty((B, L, D), dtype=torch.bfloat16).pin_memory()
-    to_host_value = time_e2e(e2e_steps, h_emb)
+    to_host_value = time_e2e(steps, h_emb)
     del h_emb
     e2e = {"value": max(pipe_value, sync_value), "unit": "tokens/s", "h2d_bytes_per_step": T * 8, "d2h_bytes_per_step": T * 5,
            "api": "EmbeddingCache.host_pipeline() (pipelined) / EmbeddingCache.lookup() (synchronous)",
            "mode": "pipelined (4 slots, up to 3 batches in flight)" if pipe_value >= sync_value else "synchronous call per step",
            "pipelined": pipe_value, "synchronous": sync_value,
-           "embeds_to_host": {"value": to_host_value, "unit": "tokens/s", "d2h_bytes_per_step": T * 5 + T * D * 2, "steps": e2e_steps,
+           "embeds_to_host": {"value": to_host_value, "unit": "tokens/s", "d2h_bytes_per_step": T * 5 + T * D * 2, "steps": steps,
                               "note": "synchronous lookup() per step with the [B, L, D] embeddings ALSO copied to pinned host memory: "
                                       "host-link bound"},
            "note": "ids from pinned host memory; fgram_id + match_len read back to pinned host memory every step; the embeddings "
@@ -451,6 +484,8 @@ def run_ours(args, w, rank, local_rank, world, name, steps=None):
 
     if rank != 0:
         return None
+    if snap is not None:
+        _dump_outputs(snap, dump_dir)
 
     # ---- in-run parity: two rows of batch 0 through the drop-in class against the oracle ---------------------------------
     parity = None
@@ -631,7 +666,7 @@ def run_sharded(args, w, rank, local_rank, world, modes=("peer", "nccl"), parity
 
     B, L, D, V = w["B"], w["L"], w["D"], w["V"]
     T = B * L
-    steps = max(3, min(args.steps, 20))
+    steps = args.steps
     rows_per_gpu = args.rows_per_gpu or w["N"]
     N = rows_per_gpu * world
     t_build = time.perf_counter()
@@ -799,7 +834,7 @@ def run_host(args, w, rank, local_rank, world):
     dev = torch.device("cuda", local_rank)
     B, L, D, V = w["B"], w["L"], w["D"], w["V"]
     T = B * L
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     stride, _ = sb.table_layout(w["quant"], D)
     total_ram = os.sysconf("SC_PAGE_SIZE") * os.sysconf("SC_PHYS_PAGES")
     avail = total_ram
@@ -875,14 +910,13 @@ def run_host(args, w, rank, local_rank, world):
     if not args.no_staged:
         from scone_b200.offload import StagedHostLookup
         staged = StagedHostLookup(index, table, base, micro_batches=8, max_positions=T)
-        n_st = 3
         staged.lookup(batches[0], out=out)
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        for k in range(n_st):
+        for k in range(steps):
             staged.lookup(batches[k % 4], out=out)
         torch.cuda.synchronize()
-        st_s = (time.perf_counter() - t0) / n_st
+        st_s = (time.perf_counter() - t0) / steps
         staged_info = {"value": T / st_s, "unit": "tokens/s", "host_link_GBps": hit * T * stride / st_s / 1e9, "micro_batches": 8,
                        "host_threads": staged.threads, "ms_per_step": st_s * 1e3,
                        "note": "match on the GPU, host threads gather the rows into pinned staging, cudaMemcpyAsync on a side stream, "
@@ -913,10 +947,10 @@ def run_host(args, w, rank, local_rank, world):
 # The suite
 # ------------------------------------------------------------------------------------------------------------
 
-def _child(args, name, steps, extra=(), timeout_s=600):
+def _child(args, name, extra=(), timeout_s=600):
     """Run one workload in a child process of this script (its own CUDA context: a failure or a large footprint there cannot
     take the headline line down) and return its parsed JSON line reduced to what the parent reports."""
-    cmd = [sys.executable, os.path.abspath(__file__), "--workload", name, "--steps", str(steps), "--warmup", str(args.warmup),
+    cmd = [sys.executable, os.path.abspath(__file__), "--workload", name, "--steps", str(args.steps), "--warmup", str(args.warmup),
            "--no-cpu-baseline"] + list(extra)
     t0 = time.perf_counter()
     try:
@@ -937,7 +971,7 @@ def _child(args, name, steps, extra=(), timeout_s=600):
 
 def run_suite(args, rank, local_rank, world):
     t_start = time.perf_counter()
-    line = run_ours(args, WORKLOADS["config2"], rank, local_rank, world, "config2")
+    line = run_ours(args, WORKLOADS["config2"], rank, local_rank, world, "config2", dump_dir=args.dump_outputs)
     if world == 1:
         if not args.no_configs:
             import torch
@@ -945,9 +979,9 @@ def run_suite(args, rank, local_rank, world):
             # the whole default run must end within a few minutes: each child gets what is left of `--suite-seconds`
             left = lambda: max(30.0, args.suite_seconds - (time.perf_counter() - t_start))
             configs = {}
-            configs["config1"] = _child(args, "config1", args.steps, timeout_s=min(180.0, left()))
-            configs["config3"] = _child(args, "config3", max(3, min(args.steps, 20)), timeout_s=min(300.0, left()))
-            configs["config5"] = _child(args, "config5", 10, timeout_s=min(400.0, left()))
+            configs["config1"] = _child(args, "config1", timeout_s=min(180.0, left()))
+            configs["config3"] = _child(args, "config3", timeout_s=min(300.0, left()))
+            configs["config5"] = _child(args, "config5", timeout_s=min(400.0, left()))
             line["configs"] = configs
             line["suite_seconds"] = time.perf_counter() - t_start
         print(json.dumps(line), flush=True)
@@ -968,7 +1002,7 @@ def run_suite(args, rank, local_rank, world):
         # config 3 is named "on 1 and 8xB200": its 21 GB table fits every GPU, so at N > 1 it is N replicas with their own batches
         t0 = time.perf_counter()
         try:
-            c3 = run_ours(args, WORKLOADS["config3"], rank, local_rank, world, "config3", steps=max(3, min(args.steps, 20))) or {}
+            c3 = run_ours(args, WORKLOADS["config3"], rank, local_rank, world, "config3") or {}
             c3 = {k: c3.get(k) for k in ("value", "unit", "ms_per_step", "steps", "dtype", "gpu_launches", "clocks", "roofline", "e2e", "parity",
                                          "config") if c3.get(k) is not None}
         except Exception as e:
@@ -999,7 +1033,7 @@ def run_suite(args, rank, local_rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps of every measurement, child configs included")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="suite", choices=["suite"] + sorted(WORKLOADS))
@@ -1017,7 +1051,13 @@ def main():
     ap.add_argument("--sharded-mode", default="both", choices=["both", "peer", "nccl"], help="config4: which exchange variants to run")
     ap.add_argument("--nccl-micro", type=int, default=1, help="config4, NCCL variant: micro-batches the two all-to-alls are pipelined over")
     ap.add_argument("--host-fraction", type=float, default=0.0, help="config5: fraction of host RAM to pin (default 0.5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/*.npy (suite headline and config1..config3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or WORKLOADS.get(args.workload, {}).get("tier")):
+        ap.error("--dump-outputs applies to the GPU suite and to config1..config3")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -1043,7 +1083,7 @@ def main():
     elif w.get("tier") == "host":
         print(json.dumps(run_host(args, w, rank, local_rank, world)), flush=True)
     else:
-        line = run_ours(args, w, rank, local_rank, world, args.workload)
+        line = run_ours(args, w, rank, local_rank, world, args.workload, dump_dir=args.dump_outputs)
         if rank == 0:
             print(json.dumps(line), flush=True)
         if world > 1:
@@ -1052,4 +1092,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
     main()

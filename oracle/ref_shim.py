@@ -1,9 +1,10 @@
-"""Import the UNMODIFIED reference classes from /root/reference (authoring container only).
+"""Import the UNMODIFIED reference classes from a checkout of the upstream project: oracle/_ref (git-ignored), or the
+directory SCONE_REFERENCE_ROOT names.
 
-TEST INFRASTRUCTURE ONLY.  /root/reference does not exist on the GPU box, so
+TEST INFRASTRUCTURE ONLY.  The reference is not part of this repository, so
 nothing in ``-m gpu`` tests, ``smoke()`` or ``bench.py`` may call this; it is
-used by ``tests/golden/make_golden.py`` (fixture generation) and by CPU tests
-that are skipped when the reference tree is absent.
+used by ``tests/golden/make_golden.py`` (fixture generation) and by the CPU
+test that runs the reference side by side with the oracle when a checkout is present.
 
 The reference does not import cleanly as shipped: ``scone/utils/__init__.py:3``
 imports a module that does not exist (``scone.utils.cloud``), which breaks
@@ -19,7 +20,7 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("SCONE_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("SCONE_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def available() -> bool:
@@ -37,7 +38,8 @@ def _load(name: str, relpath: str):
 def load_reference():
     """Returns (NGramExtractor, EmbeddingCache) classes of the reference."""
     if not available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference checkout not found at {REFERENCE_ROOT}: put the upstream scone repository there or "
+                           "name it in SCONE_REFERENCE_ROOT")
     # embedding_cache.py does `from scone.tokenization.n_gram_extractor import NGramExtractor`.
     # Provide bare package shells (no __init__ executed) so that import resolves
     # to the file we load by path.

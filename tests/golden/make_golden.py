@@ -1,11 +1,14 @@
-"""Generate golden fixtures by running the UNMODIFIED reference (authoring container only).
+"""Generate golden fixtures by running the UNMODIFIED reference.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [fixture ...]      (default: all of them)
 
-Imports ``NGramExtractor`` / ``EmbeddingCache`` from /root/reference through
+The reference is read from oracle/_ref (a git-ignored checkout of the upstream
+project) or from the directory SCONE_REFERENCE_ROOT names.
+
+Imports ``NGramExtractor`` / ``EmbeddingCache`` from that checkout through
 ``oracle/ref_shim.py`` and records their outputs on seeded inputs into small
-``.npz`` files next to this script.  The GPU box has no /root/reference, so
-the tests read only the committed ``.npz`` files.
+``.npz`` files next to this script.  The reference is not part of this
+repository, so the tests read only the committed ``.npz`` files.
 
 What each fixture pins (reference file:line):
   kat0.npz        fit + longest match on the hand-sized case of SURVEY.md 8c
@@ -23,6 +26,9 @@ What each fixture pins (reference file:line):
                   memmap backends, embedding_cache.py:56-147), `.half()` of the
                   gathered rows (engine.py:265-266), and the engine's assemble
                   loop (engine.py:235-259) re-enacted on the reference objects
+  live_2024.npz   fit (max_n = 4, min_freq = 2, max_f_grams = 500) on a 30-text Zipf(1.2)
+                  corpus over 60 tokens and get_token_f_grams of a 120-token query
+                  (tests/test_oracle.py::test_live_reference_agrees_with_oracle)
 """
 
 from __future__ import annotations
@@ -234,12 +240,27 @@ def make_cache_small():
                         te_pos=te_pos, te_cnt=te_cnt, te_rows=te_rows, fgram_id=fid, match_len=ml)
 
 
+def make_live_2024():
+    """The inputs of test_live_reference_agrees_with_oracle, drawn the same way there."""
+    rng = np.random.default_rng(2024)
+    corpus = [((rng.zipf(1.2, size=80) - 1) % 60).tolist() for _ in range(30)]
+    q = ((rng.zipf(1.2, size=120) - 1) % 60).tolist()
+    max_n, min_freq, max_f = 4, 2, 500
+    ex = NGramExtractor(max_n=max_n, min_freq=min_freq, max_f_grams=max_f).fit(corpus, verbose=False)
+    toks, lens = vocab_arrays(ex, max_n)
+    offs, flat = ref_containing(ex, q)
+    np.savez_compressed(os.path.join(HERE, "live_2024.npz"), corpus=np.array(corpus, dtype=np.int64), query=np.array(q, dtype=np.int64),
+                        max_n=max_n, min_freq=min_freq, max_f_grams=max_f, vocab_tokens=toks, vocab_lens=lens,
+                        cont_offs=offs, cont_flat=flat)
+
+
+FIXTURES = {"kat0": make_kat0, "fit_small": make_fit_small, "fit_medium": make_fit_medium, "vocab_n5": make_vocab_n5,
+            "cache_small": make_cache_small, "live_2024": make_live_2024}
+
+
 if __name__ == "__main__":
-    make_kat0()
-    make_fit_small()
-    make_fit_medium()
-    make_vocab_n5()
-    make_cache_small()
+    for name in sys.argv[1:] or list(FIXTURES):
+        FIXTURES[name]()
     for f in sorted(os.listdir(HERE)):
         if f.endswith(".npz"):
             print(f, os.path.getsize(os.path.join(HERE, f)), "bytes")

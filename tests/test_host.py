@@ -253,6 +253,54 @@ def test_bench_reference_arm_runs_on_cpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--workload", "config1",
                           "--steps", "1", "--warmup", "0"], capture_output=True, text=True, timeout=120, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+    # the dump belongs to the GPU arm, and a run needs at least one timed step
+    for extra in (["--impl", "reference", "--dump-outputs", "x"], ["--workload", "config5", "--dump-outputs", "x"], ["--steps", "0"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120)
+        assert out.returncode == 2 and "error" in out.stderr
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the results of the last timed step as float32 / float64 within 64 MB.  The steps
+    rotate over 8 seeded id batches (step k runs batch k % 8), so 2 and 10 steps both end on batch 1 and 1 step on batch 0:
+    the first two dumps are identical, the third differs, and batch 1's dump is checked against the oracle on inputs rebuilt
+    here from bench.py's seeds (vocabulary seed 0, table seed 2, fallback rows seed 3, batch k seed 100 + k)."""
+    import subprocess
+    import sys
+    from oracle.c_oracle import COracleIndex
+    from scone_b200.utils import synthetic as S
+    dumps = {}
+    for steps in ("2", "10", "1"):
+        d = tmp_path / steps
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "config1", "--steps", steps, "--warmup", "1",
+                              "--no-cpu-baseline", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert sorted(os.listdir(d)) == ["embeddings.npy", "fgram_id.npy", "match_len.npy"]
+        assert sum(os.path.getsize(d / f) for f in os.listdir(d)) <= 64 << 20
+        dumps[steps] = {f[:-4]: np.load(d / f) for f in os.listdir(d)}
+    z = dumps["2"]
+    assert z["fgram_id"].dtype == np.float64 and z["match_len"].dtype == np.float32 and z["embeddings"].dtype == np.float32
+    assert z["fgram_id"].shape == z["match_len"].shape == (8, 512) and z["embeddings"].shape == (8 * 512, 768)
+    for k in z:
+        assert np.array_equal(z[k], dumps["10"][k]), k
+    assert not np.array_equal(z["fgram_id"], dumps["1"]["fgram_id"])
+    # config1: N = 100 000 f-grams, max_n = 3, V = 50 257, D = 768, FP16 table, batch 8 x 512, bf16 output
+    N, max_n, V, D, B, L = 100_000, 3, 50_257, 768, 8, 512
+    toks, lens, longest = S.make_vocab_device(N, max_n, V, seed=0, device="cuda", return_longest=True)
+    q = S.make_stream_device(toks, lens, B, L, V, seed=101, p_plant=1.0, pick_ids=longest).cpu().numpy()
+    wid, wlen = COracleIndex(toks.cpu().numpy(), lens.cpu().numpy()).match(q, nthreads=4)
+    assert (wid >= 0).any() and (wid < 0).any()
+    assert np.array_equal(z["fgram_id"], wid) and np.array_equal(z["match_len"], wlen)
+    gen = torch.Generator(device="cuda")
+    gen.manual_seed(2)
+    rows = torch.randn((N, D), generator=gen, device="cuda", dtype=torch.float32) * 0.02
+    hit = wid >= 0
+    want = np.empty((B, L, D), np.uint16)
+    want[hit] = po.cast_bits(po.OracleTable.from_fp32(rows[torch.from_numpy(wid[hit].astype(np.int64)).cuda()].cpu().numpy(), "fp16")
+                             .rows_fp32(np.arange(int(hit.sum()))), "bf16")
+    base = S.make_base_device(V, D, torch.bfloat16, seed=3, device="cuda").view(torch.int16).cpu().numpy().view(np.uint16)
+    want[~hit] = base[q[~hit]]
+    assert np.array_equal(z["embeddings"], po.bf16_bits_to_f32(want).reshape(B * L, D))
 
 
 def test_extractor_map_assignment_like_reference_load():

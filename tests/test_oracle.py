@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import load_golden, vocab_dict
+from conftest import GOLDEN, load_golden, vocab_dict
 from oracle import py_oracle as po
 from oracle import ref_shim
 from oracle.c_oracle import COracleIndex, lib as c_lib
@@ -124,17 +124,33 @@ def test_fuzz_py_vs_c_oracle():
         assert np.array_equal(a[0], c[0]) and np.array_equal(a[1], c[1])
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
-def test_live_reference_agrees_with_oracle():
-    """In the authoring container: run the unmodified reference side by side on fresh random input."""
-    NGramExtractor, EmbeddingCache = ref_shim.load_reference()
+def _live_corpus_and_query():
     rng = np.random.default_rng(2024)
     corpus = [((rng.zipf(1.2, size=80) - 1) % 60).tolist() for _ in range(30)]
-    ex = NGramExtractor(max_n=4, min_freq=2, max_f_grams=500).fit(corpus, verbose=False)
+    return corpus, ((rng.zipf(1.2, size=120) - 1) % 60).tolist()
+
+
+@pytest.mark.skipif(not (os.path.exists(os.path.join(GOLDEN, "live_2024.npz")) or ref_shim.available()),
+                    reason="needs tests/golden/live_2024.npz or a reference checkout (see tests/golden/make_golden.py)")
+def test_live_reference_agrees_with_oracle():
+    """fit and get_token_f_grams of the unmodified reference on one more seeded corpus and query: against its output stored
+    by tests/golden/make_golden.py, and side by side with the reference itself when a checkout is present."""
+    corpus, q = _live_corpus_and_query()
     grams = po.fit(corpus, 4, 2, 500)
-    assert grams == [ex.id_to_f_gram[i] for i in range(len(grams))] and len(grams) == len(ex.f_grams)
-    q = ((rng.zipf(1.2, size=120) - 1) % 60).tolist()
-    assert po.token_f_grams(ex.f_grams, 4, q) == ex.get_token_f_grams(q)
+    tf = po.token_f_grams(set(grams), 4, q)
+    if os.path.exists(os.path.join(GOLDEN, "live_2024.npz")):
+        z = load_golden("live_2024.npz")
+        assert np.array_equal(z["corpus"], corpus) and np.array_equal(z["query"], q)
+        assert grams == [tuple(int(t) for t in z["vocab_tokens"][i, :z["vocab_lens"][i]]) for i in range(len(z["vocab_lens"]))]
+        g2i = {g: i for i, g in enumerate(grams)}
+        offs = z["cont_offs"]
+        for pos in range(len(q)):
+            assert [g2i[g] for g in tf[pos]] == z["cont_flat"][offs[pos]:offs[pos + 1]].tolist()
+    if ref_shim.available():
+        NGramExtractor, EmbeddingCache = ref_shim.load_reference()
+        ex = NGramExtractor(max_n=4, min_freq=2, max_f_grams=500).fit(corpus, verbose=False)
+        assert grams == [ex.id_to_f_gram[i] for i in range(len(grams))] and len(grams) == len(ex.f_grams)
+        assert tf == ex.get_token_f_grams(q)
 
 
 # ---- rows: gather, fp16 cast, quant formulas ---------------------------------------------------

@@ -9,7 +9,7 @@ import ctypes as C
 import os
 
 PKG = os.path.dirname(os.path.abspath(__file__))
-# SCONE_B200_LIB: another build of the library (development: the SCONE_TUNE build, A/B against an older build)
+# SCONE_B200_LIB: another build of the library (development: same-box A/B against an older build)
 LIB_PATH = os.environ.get("SCONE_B200_LIB") or os.path.join(PKG, "lib", "libscone_b200.so")
 
 QUANT = {"fp16": 0, "int8": 1, "int4": 2, "fp32": 3}

@@ -15,9 +15,7 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.path.join(PKG, "lib")
-# SCONE_TUNE=1 builds the development library (extra kernel shapes for tools/tune_*.py) next to the product one
-TUNE = bool(os.environ.get("SCONE_TUNE"))
-LIB_PATH = os.path.join(LIB_DIR, "libscone_b200_tune.so" if TUNE else "libscone_b200.so")
+LIB_PATH = os.path.join(LIB_DIR, "libscone_b200.so")
 SOURCES = ["api.cu", "index.cu", "table.cu", "embed.cu", "pipeline.cu", "fold.cu", "fit.cu"]
 # the fused path's kernels are compiled once per (table format, output type): eight translation units, in parallel
 INST_SOURCE = "embed_inst.cu"
@@ -60,11 +58,10 @@ def build(force: bool = False, verbose: bool = False) -> str:
         return LIB_PATH
     from concurrent.futures import ThreadPoolExecutor
     os.makedirs(LIB_DIR, exist_ok=True)
-    obj_dir = os.path.join(LIB_DIR, "obj_tune" if TUNE else "obj")
+    obj_dir = os.path.join(LIB_DIR, "obj")
     os.makedirs(obj_dir, exist_ok=True)
     nvcc = nvcc_path()
-    tune = ["-DSCONE_TUNE"] if TUNE else []      # extra kernel variants for tools/tune_embed.py
-    common = [nvcc] + NVCC_FLAGS + tune + (["-Xptxas", "-v"] if verbose else [])
+    common = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else [])
     jobs = []
     for q, o in INSTANCES:                                                 # the long ones first
         obj = os.path.join(obj_dir, f"embed_inst_q{q}_{o}.o")

@@ -109,9 +109,6 @@ struct IndexView {
     int32_t compact;
     const uint32_t *filter;  // NULL = probe every candidate
     uint32_t filter_mask;    // number of filter words
-#ifdef SCONE_TUNE
-    const uint8_t *hint;  // development only, see match.cuh
-#endif
 };
 
 // Batches below this many positions are latency-bound: the filter's extra L2 round trip costs more than the probes it saves.

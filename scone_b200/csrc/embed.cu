@@ -3,6 +3,8 @@
 // Takes over, per position, get_token_f_grams + f_gram_to_id + get_embeddings + the engine's assemble loop + the wte
 // fallback of the reference (scone/tokenization/n_gram_extractor.py:106-126, scone/inference/embedding_cache.py:149-181,
 // scone/inference/engine.py:235-266, scone/models/language_model.py:239-243), with Algorithm-2 semantics.
+#include <cstdlib>
+
 #include "embed_kernels.cuh"
 
 namespace scone {
@@ -40,12 +42,6 @@ static int dispatch(int P, EmbedParams &p, int quant, int out_dtype, cudaStream_
     const int *order = moved >= 6144 ? wide : narrow;
     const int n_order = 4;
     int rc = kNoFit;
-#ifdef SCONE_TUNE
-    if (const char *e = getenv("SCONE_EMBED_P")) P = atoi(e) > P ? atoi(e) : P;
-    if (const char *e = getenv("SCONE_STAGGER_NS")) p.stagger_ns = atoi(e);
-    if (const char *e = getenv("SCONE_STAGGER_CTA_NS")) p.stagger_cta_ns = atoi(e);
-    if (const char *e = getenv("SCONE_BASE_POLICY")) p.base_policy = atoi(e);
-#endif
     if (p.additive && P < 4) P = 4;  // see launch_p
     // Two kernels (measured, profiles/tune_r02.md): the plain path runs fastest on embed_bulk_kernel (one ring, the matcher
     // stages its own tile: fewest hand-offs); with extra rows per position (fused position add, additive combine) the
@@ -107,19 +103,6 @@ using namespace scone;
 
 extern "C" {
 
-#ifdef SCONE_TUNE
-static const int64_t *g_hint_ids = nullptr;
-static const uint8_t *g_hint = nullptr;
-static int64_t g_hint_n = 0;
-// what-if experiment: match lengths known in advance for the id buffer [ids_base, ids_base + n)
-int scone_debug_set_hint(const int64_t *d_ids_base, const uint8_t *d_match_len, int64_t n) {
-    g_hint_ids = d_ids_base;
-    g_hint = d_match_len;
-    g_hint_n = n;
-    return SCONE_OK;
-}
-#endif
-
 static int embed_forward_impl(const scone_index_t *index, const scone_table_desc_t *table, const void *d_base_emb, int64_t base_rows,
                               const void *d_pos_emb, const int64_t *d_ids, int64_t B, int64_t L, void *d_out, int32_t out_dtype,
                               int32_t *d_out_id, uint8_t *d_out_len, uint32_t *d_status, void *stream_, uint32_t flags) {
@@ -153,11 +136,7 @@ static int embed_forward_impl(const scone_index_t *index, const scone_table_desc
     p.out_len = d_out_len;
     p.status = d_status;
     p.additive = (flags & SCONE_EMBED_ADDITIVE) ? 1 : 0;
-    static const bool no_early = getenv("SCONE_NO_EARLY") != nullptr;  // A/B switch: ignore SCONE_EMBED_INPUTS_STABLE
-    p.flags = no_early ? (flags & ~SCONE_EMBED_INPUTS_STABLE) : flags;
-#ifdef SCONE_TUNE
-    if (g_hint && getenv("SCONE_HINT") && d_ids >= g_hint_ids && d_ids + T <= g_hint_ids + g_hint_n) p.ix.hint = g_hint + (d_ids - g_hint_ids);
-#endif
+    p.flags = flags;
     return dispatch(lanes_per_position(ix->len_mask, ix->max_n), p, table->quant, out_dtype, stream);
 }
 

@@ -20,11 +20,3 @@ int SCONE_INST_NAME(SCONE_INST_QUANT, SCONE_INST_OUT)(int P, EmbedParams &p, cud
 }
 
 }  // namespace scone
-
-#if defined(SCONE_TUNE) && SCONE_INST_QUANT == SCONE_QUANT_INT8 && SCONE_INST_OUT == SCONE_OUT_BF16
-// development only (tools/timeline.py): the stamps of the INT8 -> bf16 instance (config 2)
-extern "C" int scone_debug_timeline(unsigned long long *out16) {
-    SCONE_CUDA(cudaMemcpyFromSymbol(out16, scone::g_timeline, sizeof(unsigned long long) * 16));
-    return SCONE_OK;
-}
-#endif

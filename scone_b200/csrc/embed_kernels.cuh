@@ -26,8 +26,6 @@
 //
 // This header is compiled once per (table format, output type) by embed_inst.cu; embed.cu holds dispatch and the C ABI.
 #pragma once
-#include <cstdlib>
-
 #include "common.cuh"
 #include "match.cuh"
 
@@ -56,9 +54,7 @@ struct EmbedParams {
     int32_t world;        // 1 = the whole table is at `rows`
     int32_t additive;     // 1 = reference-code combine: base row + table row on a hit (language_model.py:239-243)
     int32_t stagger_ns;   // matcher warp w starts its first probes w * stagger_ns later (0 = together)
-    int32_t stagger_cta_ns;  // ... and the c-th CTA of an SM (blockIdx / #SMs) another c * stagger_cta_ns later
-    uint32_t flags;          // SCONE_EMBED_* of scone_embed_opts_t
-    int32_t base_policy;     // L2 policy of the fallback / base rows: 0 evict-first (streamed), 1 default, 2 evict-last (kept)
+    uint32_t flags;       // SCONE_EMBED_* of scone_embed_opts_t
 };
 
 // row bytes holding 8 consecutive elements of a stored row
@@ -78,15 +74,6 @@ __device__ __forceinline__ const uint8_t *row_ptr(const EmbedParams &p, int32_t 
 
 constexpr int kRing = 16;  // tiles the matchers may run ahead of the gather warps
 constexpr uint32_t kEmbedPipe = 1u << 31;  // EmbedParams::flags, internal: use embed_pipe_kernel instead of embed_bulk_kernel
-
-// L2 policy for the fallback / base rows (EmbedParams::base_policy)
-__device__ __forceinline__ uint64_t base_row_policy(int which) {
-    uint64_t pol;
-    if (which == 2) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-    else if (which == 1) asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
-    else asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
 
 // programmatic dependent launch: block until the grid this one was launched behind has completed and its writes are visible
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -412,21 +399,6 @@ __device__ __forceinline__ void stream_from_smem(const EmbedParams &p, const uin
     }
 }
 
-#ifdef SCONE_TUNE
-// development only: nanosecond stamps of block 0 (slots 0-7) and the last block (8-15), read by tools/timeline.py
-static __device__ unsigned long long g_timeline[16];  // one copy per translation unit (embed_inst.cu)
-__device__ __forceinline__ void stamp(int k) {
-    if (blockIdx.x == 0 || blockIdx.x == gridDim.x - 1) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        g_timeline[(blockIdx.x == 0 ? 0 : 8) + k] = t;
-    }
-}
-#define SCONE_STAMP(k, cond) do { if (cond) stamp(k); } while (0)
-#else
-#define SCONE_STAMP(k, cond) do { } while (0)
-#endif
-
 constexpr int kMaxRing = 16;
 // bytes of barriers + ring metadata in front of the row slots
 __host__ __device__ constexpr int bulk_header_bytes(int G) { return (2 * kMaxRing * 8 + kMaxRing * G * 8 + 127) / 128 * 128; }
@@ -464,13 +436,11 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
     const bool early = (p.flags & SCONE_EMBED_INPUTS_STABLE) != 0;
     bool waited = !early;
     if (!early) griddep_wait();
-    SCONE_STAMP(0, threadIdx.x == 0);
 
     if (warp < NM) {
         const int j = lane / P;
         const int back = p.ix.max_n - 1;
         const uint64_t pol = policy_evict_first();
-        const uint64_t pol_base = base_row_policy(p.base_policy);
         int64_t it = warp;
         int64_t tile = blockIdx.x + it * gridDim.x;
         int32_t wtok = -1;
@@ -478,7 +448,7 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
         // The first probes of all matchers of all CTAs would hit the index as one burst of random 64-byte reads; spreading
         // them lets the first tiles resolve (and their rows start to flow) before the burst has drained.
         if (!p.fgram_in) {
-            const unsigned wait_ns = (unsigned)(warp * p.stagger_ns) + (unsigned)((blockIdx.x / kNumSMsB200) * p.stagger_cta_ns);
+            const unsigned wait_ns = (unsigned)(warp * p.stagger_ns);
             if (wait_ns) __nanosleep(wait_ns);
         }
         for (; tile < p.num_tiles; it += NM, tile += (int64_t)NM * gridDim.x) {
@@ -499,9 +469,7 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
                 }
             } else {
                 if (ntile < p.num_tiles) ntok = load_window_token<P>(p.ids, p.T, ntile * G, lane, back);
-                SCONE_STAMP(1, warp == 0 && lane == 0 && it == 0 && wtok != -12345);   // ids of the first tile have arrived
                 const WindowMatch m = match_window<P>(p.ix, wtok, p.T, p.L, base, lane, back);
-                SCONE_STAMP(2, warp == 0 && lane == 0 && it == 0 && m.fid != -12345);  // first tile resolved
                 fid = m.fid;
                 mlen = m.len;
                 tok = own_token<P>(wtok, lane, back);
@@ -542,10 +510,9 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
             if (lane == 0) mbar_arrive_expect_tx(&full_bar[q], total);
             __syncwarp();
             uint8_t *slot = rows_smem + (size_t)(q * G + j) * lay.slot_bytes;
-            if (bytes) bulk_g2s(slot, src, bytes, &full_bar[q], fid >= 0 ? pol : pol_base);
+            if (bytes) bulk_g2s(slot, src, bytes, &full_bar[q], pol);
             if (src2) bulk_g2s(slot + lay.pos_off, src2, (uint32_t)p.D * 2u, &full_bar[q], policy_evict_last());
-            if (src3) bulk_g2s(slot + add_off, src3, (uint32_t)p.D * 2u, &full_bar[q], pol_base);
-            SCONE_STAMP(3, warp == 0 && lane == 0 && it == 0);                        // first bulk copies issued
+            if (src3) bulk_g2s(slot + add_off, src3, (uint32_t)p.D * 2u, &full_bar[q], pol);
             // the match result is this warp's only global write: after the previous grid (see `early` above)
             if (!waited) {
                 griddep_wait();
@@ -556,7 +523,6 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
                 if (p.out_len) p.out_len[i] = (uint8_t)mlen;
             }
         }
-        SCONE_STAMP(7, warp == 0 && lane == 0);                                       // matcher 0 done
     } else {
         // every gather warp waits for and releases every tile, in order (see embed_kernel)
         bool flagged = false;
@@ -566,7 +532,6 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
         for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++itl) {
             const int q = (int)(itl % R);
             mbar_wait(&full_bar[q], (uint32_t)((itl / R) & 1));
-            SCONE_STAMP(4, w == 0 && lane == 0 && itl == 0);                          // first rows have landed
             if (!waited) {  // rows are staged; the stores below are the first thing that must follow the previous grid
                 griddep_wait();
                 waited = true;
@@ -605,45 +570,38 @@ static int num_sms() {
     return n;
 }
 
-// Tuning hook (tools/tune_embed.py): SCONE_EMBED_VARIANT="kind:U:NM:NG:MINB:smemKB" (kind 0 = register loads,
-// 1 = bulk copies) selects another instantiation for the combinations compiled under -DSCONE_TUNE.
-struct Variant {
-    int kind = -1, u = 0, nm = 0, ng = 0, minb = 0, smem_kb = 0;
-};
-static Variant variant() {
-    Variant v;
-    if (const char *e = getenv("SCONE_EMBED_VARIANT")) sscanf(e, "%d:%d:%d:%d:%d:%d", &v.kind, &v.u, &v.nm, &v.ng, &v.minb, &v.smem_kb);
-    return v;
-}
-
-// Kernels are launched with programmatic stream serialization (PDL): back-to-back steps overlap this kernel's launch
+// Launches kern(p[, lay]) as a persistent grid over the call's tiles of G positions: at most MINB CTAs per SM, `smem` bytes
+// of dynamic shared memory.  Kernels are launched with programmatic stream serialization (PDL): back-to-back steps overlap this kernel's launch
 // and prologue (barrier init) with the previous kernel's tail; its griddepcontrol.wait still orders everything it reads
 // or writes after the previous grid.  Same-box A/B on B200: config 1 -8 %, config 2 -1.6 %, config 3 unchanged.
-// SCONE_NO_PDL=1 falls back to plain launches (the griddepcontrol instructions are then no-ops).
-template <typename Kern, typename... Args>
-static int launch_pdl(Kern kern, unsigned blocks, unsigned threads, size_t smem, cudaStream_t stream, Args... args) {
-    static const bool no_pdl = getenv("SCONE_NO_PDL") != nullptr;
+template <auto kern, int G, int MINB, typename... Layout>
+static int launch_resident(EmbedParams &p, unsigned threads, int smem, cudaStream_t stream, Layout... lay) {
+    static int configured[64] = {0};  // per device: the attribute lives in the device's context
+    int dev = 0;
+    SCONE_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 64 || configured[dev] < smem) {
+        SCONE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        if (dev >= 0 && dev < 64) configured[dev] = smem;
+    }
+    p.num_tiles = (p.T + G - 1) / G;
+    const int64_t resident = (int64_t)num_sms() * MINB;
     cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(blocks);
+    cfg.gridDim = dim3((unsigned)(p.num_tiles < resident ? p.num_tiles : resident));
     cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = smem;
+    cfg.dynamicSmemBytes = (size_t)smem;
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    SCONE_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
+    cfg.numAttrs = 1;
+    SCONE_CUDA(cudaLaunchKernelEx(&cfg, kern, p, lay...));
     return SCONE_OK;
 }
 
 template <int QUANT, int OUT, int P, int U, int NM, int NG, int MINB>
 static int launch_ldg(EmbedParams &p, cudaStream_t stream) {
-    constexpr int G = 32 / P;
-    p.num_tiles = (p.T + G - 1) / G;
-    const int64_t resident = (int64_t)num_sms() * MINB;
-    const unsigned blocks = (unsigned)(p.num_tiles < resident ? p.num_tiles : resident);
-    return launch_pdl(embed_kernel<QUANT, OUT, P, U, NM, NG, MINB>, blocks, 32 * (NM + NG), 0, stream, p);
+    return launch_resident<embed_kernel<QUANT, OUT, P, U, NM, NG, MINB>, 32 / P, MINB>(p, 32 * (NM + NG), 0, stream);
 }
 
 // Ring geometry for the bulk variant; returns false when rows are too wide for the budget.
@@ -674,39 +632,14 @@ static bool bulk_layout(const EmbedParams &p, int G, int nm, int budget_bytes, B
 
 template <int QUANT, int OUT, int P, int NM, int NG, int MINB, bool ADD>
 static int launch_bulk(EmbedParams &p, const BulkLayout &lay, cudaStream_t stream) {
-    constexpr int G = 32 / P;
-    auto kern = embed_bulk_kernel<QUANT, OUT, P, NM, NG, MINB, ADD>;
-    if (p.stagger_ns < 0) p.stagger_ns = 0;  // "off" from a SCONE_TUNE override on a shape that does not stagger
-    static int configured[64] = {0};  // per device: the attribute lives in the device's context
-    int dev = 0;
-    SCONE_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64 || configured[dev] < lay.smem_bytes) {
-        SCONE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, lay.smem_bytes));
-        if (dev >= 0 && dev < 64) configured[dev] = lay.smem_bytes;
-    }
-    p.num_tiles = (p.T + G - 1) / G;
-    const int64_t resident = (int64_t)num_sms() * MINB;
-    const unsigned blocks = (unsigned)(p.num_tiles < resident ? p.num_tiles : resident);
-    return launch_pdl(kern, blocks, 32 * (NM + NG), (size_t)lay.smem_bytes, stream, p, lay);
+    return launch_resident<embed_bulk_kernel<QUANT, OUT, P, NM, NG, MINB, ADD>, 32 / P, MINB>(p, 32 * (NM + NG), lay.smem_bytes, stream, lay);
 }
 
 template <int QUANT, int OUT, int P, int NM, int NL, int NG, int MINB, bool ADD>
 static int launch_pipe(EmbedParams &p, const PipeLayout &lay, cudaStream_t stream) {
     constexpr int G = 32 / P;
     static_assert(NL <= G, "a loader without a position");
-    auto kern = embed_pipe_kernel<QUANT, OUT, P, NM, NL, NG, MINB, ADD>;
-    if (p.stagger_ns < 0) p.stagger_ns = 0;  // "off" from a SCONE_TUNE override on a shape that does not stagger
-    static int configured[64] = {0};  // per device: the attribute lives in the device's context
-    int dev = 0;
-    SCONE_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64 || configured[dev] < lay.smem_bytes) {
-        SCONE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, lay.smem_bytes));
-        if (dev >= 0 && dev < 64) configured[dev] = lay.smem_bytes;
-    }
-    p.num_tiles = (p.T + G - 1) / G;
-    const int64_t resident = (int64_t)num_sms() * MINB;
-    const unsigned blocks = (unsigned)(p.num_tiles < resident ? p.num_tiles : resident);
-    return launch_pdl(kern, blocks, 32 * (NM + NL + NG), (size_t)lay.smem_bytes, stream, p, lay);
+    return launch_resident<embed_pipe_kernel<QUANT, OUT, P, NM, NL, NG, MINB, ADD>, G, MINB>(p, 32 * (NM + NL + NG), lay.smem_bytes, stream, lay);
 }
 
 // Kernel selection (measured on B200, profiles/tune_r01.md and tune_r02.md).  Rows that fit a shared-memory ring go through
@@ -736,10 +669,6 @@ constexpr int kNoFit = 1;
 // no effect on the wide shapes; below two tiles per matcher the delay would be exposed instead.
 template <int P, int NM, int MINB>
 static void set_stagger(EmbedParams &p) {
-    if (p.stagger_ns != 0) {  // SCONE_TUNE override; negative = off
-        if (p.stagger_ns < 0) p.stagger_ns = 0;
-        return;
-    }
     constexpr int G = 32 / P;
     if ((p.T + G - 1) / G >= 2ll * NM * MINB * num_sms()) p.stagger_ns = 500;
 }
@@ -748,32 +677,6 @@ template <int QUANT, int OUT, int P, bool ADD>
 static int launch(EmbedParams &p, cudaStream_t stream, int shape) {
     constexpr int G = 32 / P;
     BulkLayout lay;
-#ifdef SCONE_TUNE
-    if constexpr (OUT == SCONE_OUT_BF16 && (P == 4 || P == 8)) {
-        const Variant v = variant();
-#define SCONE_B(NMM, NGG, MM)                                                                                               \
-    if (v.kind == 1 && v.nm == NMM && v.ng == NGG && v.minb == MM && bulk_layout(p, G, NMM, v.smem_kb * 1024, lay)) \
-        return launch_bulk<QUANT, OUT, P, NMM, NGG, MM, ADD>(p, lay, stream);
-        SCONE_B(3, 6, 3) SCONE_B(4, 8, 2) SCONE_B(6, 6, 2) SCONE_B(8, 8, 1) SCONE_B(12, 12, 1) SCONE_B(6, 10, 2) SCONE_B(4, 12, 2)
-        SCONE_B(8, 16, 1) SCONE_B(12, 20, 1) SCONE_B(3, 5, 3) SCONE_B(5, 5, 3) SCONE_B(4, 6, 3) SCONE_B(8, 12, 1) SCONE_B(6, 18, 1)
-        SCONE_B(4, 12, 1) SCONE_B(8, 4, 2) SCONE_B(6, 6, 3) SCONE_B(8, 6, 2) SCONE_B(5, 3, 4) SCONE_B(6, 2, 4)
-        SCONE_B(3, 12, 1) SCONE_B(6, 12, 1) SCONE_B(6, 4, 3) SCONE_B(4, 4, 3) SCONE_B(2, 6, 3) SCONE_B(2, 12, 1)
-#undef SCONE_B
-        if (v.kind == 0) return launch_ldg<QUANT, OUT, P, 4, 2, 6, 4>(p, stream);
-        // kind 2: the three-role pipeline with NM matchers (+ 1 loader) + NG gather warps
-        PipeLayout pv;
-        // (the U field of the variant string is the number of loader warps)
-#define SCONE_PV(NMM, NLL, NGG, MM)                                                                                                    \
-    if (v.kind == 2 && v.nm == NMM && v.u == NLL && v.ng == NGG && v.minb == MM && pipe_layout(p, G, NMM, v.smem_kb * 1024, pv)) \
-        return launch_pipe<QUANT, OUT, P, NMM, NLL, NGG, MM, ADD>(p, pv, stream);
-        if constexpr (P == 4) {
-            SCONE_PV(5, 1, 4, 3) SCONE_PV(6, 1, 4, 3) SCONE_PV(5, 2, 4, 3) SCONE_PV(4, 2, 4, 3) SCONE_PV(4, 2, 8, 2) SCONE_PV(4, 4, 8, 2)
-            SCONE_PV(6, 2, 8, 2) SCONE_PV(6, 4, 8, 2) SCONE_PV(6, 2, 12, 1) SCONE_PV(6, 4, 12, 1) SCONE_PV(8, 4, 12, 1) SCONE_PV(8, 4, 16, 1)
-            SCONE_PV(8, 8, 16, 1) SCONE_PV(6, 1, 12, 1) SCONE_PV(4, 4, 12, 1) SCONE_PV(8, 2, 8, 2)
-        }
-#undef SCONE_PV
-    }
-#endif
     if (p.flags & kEmbedPipe) {
         // three-role pipeline (embed_pipe.cuh): tiles keep their full size, the row ring only needs two slots
         PipeLayout pl;

@@ -132,7 +132,7 @@ __global__ void __launch_bounds__(32 * (NM + NL + NG), MINB) embed_pipe_kernel(c
     } else if (warp < NM + NL) {
         // ===== loader warps: tiles in order; lane g of loader g % NL stages position g of the tile =====
         const int ld = warp - NM;
-        const uint64_t pol = policy_evict_first(), pol_keep = policy_evict_last(), pol_base = base_row_policy(p.base_policy);
+        const uint64_t pol = policy_evict_first(), pol_keep = policy_evict_last();
         int64_t itl = 0;
         for (int64_t tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++itl) {
             const int ms = (int)(itl % MR), q = (int)(itl % R);
@@ -182,8 +182,8 @@ __global__ void __launch_bounds__(32 * (NM + NL + NG), MINB) embed_pipe_kernel(c
             __syncwarp();
             uint8_t *tile_smem = rows_smem + (size_t)q * lay.tile_bytes;
             uint8_t *slot = tile_smem + (size_t)lane * lay.slot_bytes;
-            if (bytes) bulk_g2s(slot, src, bytes, &full_bar[q], e.x >= 0 ? pol : pol_base);
-            if (src3) bulk_g2s(slot + add_off, src3, (uint32_t)p.D * 2u, &full_bar[q], pol_base);
+            if (bytes) bulk_g2s(slot, src, bytes, &full_bar[q], pol);
+            if (src3) bulk_g2s(slot + add_off, src3, (uint32_t)p.D * 2u, &full_bar[q], pol);
             if (npos) {
                 int64_t cur = pos_in_row(i0, p.L, p.T);
                 for (int j = 0; j < npos;) {  // one pass unless the tile crosses the end of a sequence

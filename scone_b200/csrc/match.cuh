@@ -73,11 +73,6 @@ __device__ __forceinline__ int32_t candidate_id(const IndexView &ix, int32_t tok
             }
         }
     }
-#ifdef SCONE_TUNE
-    // what-if experiment (tools/tune_modes.py, SCONE_HINT): a perfect pre-filter -- only the candidate whose length equals
-    // the known match length of the position is probed
-    if (ix.hint && cand && ix.hint[i] != (uint8_t)n) cand = false;
-#endif
     if (!cand) return -1;
     return probe_any(ix, hash_finish(h, n), key);
 }

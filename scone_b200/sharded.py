@@ -145,24 +145,9 @@ class ShardedEmbeddingCache:
         self.last_plan: Optional[RoutePlan] = None
 
     def lookup(self, input_ids: torch.Tensor, out: Optional[torch.Tensor] = None):
-        import os
-        import time
-        trace = os.environ.get("SCONE_SHARDED_TRACE") == "1" and input_ids.is_cuda      # development: host-clock phases with syncs
-        t_ = time.perf_counter()
-
-        def mark(name):
-            nonlocal t_
-            if trace:
-                torch.cuda.synchronize()
-                now = time.perf_counter()
-                self.trace_log.append((name, (now - t_) * 1e3))
-                t_ = now
-        self.trace_log = []
         fgram_id, match_len = self.ops.match(input_ids)
-        mark("match")
         B, L = input_ids.shape
         plan = make_plan(fgram_id, self.world, self.group, micro=self.micro_batches)
-        mark("plan")
         self.last_plan = plan
         M = plan.micro
         slot2d = plan.slot_of_position.view(B, L)
@@ -174,17 +159,12 @@ class ShardedEmbeddingCache:
             b0, b1 = plan.bounds[m][0] // L, plan.bounds[m][1] // L
             reply, work = replies[m]
             work.wait()
-            mark(f"wait a2a-2[{m}]")
-            res = self.ops.assemble(input_ids[b0:b1], reply, slot2d[b0:b1].reshape(-1), None if out is None else out[b0:b1])
-            mark(f"assemble[{m}]")
-            parts[m] = res
+            parts[m] = self.ops.assemble(input_ids[b0:b1], reply, slot2d[b0:b1].reshape(-1), None if out is None else out[b0:b1])
 
         for m in range(M):
             req, work = reqs[m]
             work.wait()
-            mark(f"wait a2a-1[{m}]")
             served = self.ops.serve(req)                                     # owner side: packed rows, no dequantisation
-            mark(f"serve[{m}]")
             replies[m] = exchange_replies(plan, served, m, self.group, async_op=True)   # crosses NVLink while ...
             if m >= 1:
                 assemble(m - 1)                                             # ... the previous micro-batch is dequantised

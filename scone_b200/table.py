@@ -74,12 +74,10 @@ class CacheTable:
 
     def _alloc_host(self, nbytes: int) -> torch.Tensor:
         """Zero-filled host memory the GPU reads in place: ``scone_host_alloc`` (huge pages, parallel first touch, registered
-        as mapped pinned memory).  ``SCONE_HOST_ALLOC=torch`` falls back to a ``pin_memory=True`` torch allocation."""
+        as mapped pinned memory)."""
         import os
         import weakref
         nbytes = max(int(nbytes), 1)
-        if os.environ.get("SCONE_HOST_ALLOC") == "torch":
-            return torch.zeros((nbytes,), dtype=torch.uint8, pin_memory=True)
         host, dev = C.c_void_p(), C.c_void_p()
         with torch.cuda.device(self.device):
             _lib.check(_lib.load().scone_host_alloc(nbytes, min(32, os.cpu_count() or 1), C.byref(host), C.byref(dev)))

@@ -786,7 +786,7 @@ def test_embed_forward_all_hits_and_all_misses():
 
 def test_cuda_graph_replay_and_pdl_give_identical_results(monkeypatch):
     """The hot call is asynchronous and capture-safe: K launches replayed from one CUDA graph (as bench.py times them)
-    reproduce the eager results bit for bit (launches use programmatic dependent launch unless SCONE_NO_PDL=1)."""
+    reproduce the eager results bit for bit (every launch uses programmatic dependent launch)."""
     sb, S = _mods()
     toks, lens = S.make_vocab_numpy(4000, 4, 500, seed=91)
     ix = _index(toks, lens)

@@ -193,6 +193,23 @@ def test_header_cites_reference_for_every_entry_point():
             assert stem in integration, sym
 
 
+def test_library_reads_only_the_path_overrides_the_gpu_tests_set():
+    """The library reads five environment variables, each forcing a kernel, slot format, filter or fold path that is otherwise
+    chosen from the inputs.  tests/test_gpu_parity.py sets every one of them to run each path; a renamed or added switch fails here."""
+    overrides = {"SCONE_EMBED_PIPE", "SCONE_INDEX_FORMAT", "SCONE_INDEX_FILTER", "SCONE_FOLD_2SM", "SCONE_FOLD_XCH"}
+    csrc = os.path.join(ROOT, "scone_b200", "csrc")
+    read = set()
+    for name in sorted(os.listdir(csrc)):
+        src = open(os.path.join(csrc, name)).read()
+        names = re.findall(r'getenv\(\s*"([^"]*)"\s*\)', src)
+        assert len(names) == src.count("getenv("), f"{name}: getenv with a name that is not a string literal"
+        read |= set(names)
+    assert read == overrides
+    parity = open(os.path.join(ROOT, "tests", "test_gpu_parity.py")).read()
+    for var in sorted(overrides):
+        assert re.search(rf'setenv\(\s*"{var}"|os\.environ\[\s*"{var}"\s*\]\s*=[^=]|\b{var}\s*=\s*"', parity), var
+
+
 def test_host_gather_rows_is_pure_host_code():
     """scone_host_gather_rows (staged offload tier) runs without a GPU: multi-threaded row gather into a staging buffer."""
     from scone_b200 import _lib

@@ -1,8 +1,7 @@
 // embed_inst.cu -- the kernel instantiations of the fused path for ONE (table format, output type) pair.
 //
-// embed_kernels.cuh holds 46 kernel shapes per pair; compiling all six pairs in one translation unit took three minutes,
-// so build.py compiles this file six times in parallel with -DSCONE_INST_QUANT=q -DSCONE_INST_OUT=o and embed.cu
-// (dispatch + C ABI) calls the six entry points below.
+// Each pair holds the kernels embed_plan.h can plan (kShapes lists them); build.py compiles this file once per pair, in
+// parallel, with -DSCONE_INST_QUANT=q -DSCONE_INST_OUT=o, and embed.cu (plan + C ABI) calls the eight entry points.
 #include "embed_kernels.cuh"
 
 #if !defined(SCONE_INST_QUANT) || !defined(SCONE_INST_OUT)
@@ -14,9 +13,9 @@
 
 namespace scone {
 
-// embed_launch_q<quant>_<out>(P, params, stream, shape): SCONE_OK, an error, or kNoFit when the shape's ring cannot hold the rows
-int SCONE_INST_NAME(SCONE_INST_QUANT, SCONE_INST_OUT)(int P, EmbedParams &p, cudaStream_t stream, int shape) {
-    return launch_p<SCONE_INST_QUANT, SCONE_INST_OUT>(P, p, stream, shape);
+// embed_launch_q<quant>_<out>(plan, params, stream): SCONE_OK or an error
+int SCONE_INST_NAME(SCONE_INST_QUANT, SCONE_INST_OUT)(const EmbedPlan &pl, EmbedParams &p, cudaStream_t stream) {
+    return launch_plan<SCONE_INST_QUANT, SCONE_INST_OUT>(pl, p, stream);
 }
 
 }  // namespace scone

@@ -21,13 +21,16 @@
 //   * everything streamed (rows, fallback rows, output) carries an L2 evict-first policy, index slots evict-last.
 //   * every gather warp waits for and releases every tile, in order: with parity-only mbarriers no waiter may be more
 //     than one phase away from the barrier's current phase.
-//   * optional extra rows per position ride in the same ring slot: the position-embedding row (fused wpe add) and, in the
-//     additive combine (template parameter ADD), the base row of a hit.
+//   * extra rows per position (fused position add, additive combine) go through the three-role pipeline of
+//     embed_pipe.cuh, or through embed_kernel where rows are too wide for a ring; embed_plan.h picks the kernel.
 //
-// This header is compiled once per (table format, output type) by embed_inst.cu; embed.cu holds dispatch and the C ABI.
+// This header is compiled once per (table format, output type) by embed_inst.cu; embed.cu holds the plan and the C ABI.
 #pragma once
 #include "common.cuh"
+#include "embed_plan.h"
 #include "match.cuh"
+
+#include <utility>
 
 namespace scone {
 
@@ -72,8 +75,7 @@ __device__ __forceinline__ const uint8_t *row_ptr(const EmbedParams &p, int32_t 
     return base + (int64_t)local * p.row_stride;
 }
 
-constexpr int kRing = 16;  // tiles the matchers may run ahead of the gather warps
-constexpr uint32_t kEmbedPipe = 1u << 31;  // EmbedParams::flags, internal: use embed_pipe_kernel instead of embed_bulk_kernel
+constexpr int kRing = 16;  // tiles embed_kernel's matchers may run ahead of the gather warps
 
 // programmatic dependent launch: block until the grid this one was launched behind has completed and its writes are visible
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -202,6 +204,46 @@ __device__ __noinline__ void stream_general(const EmbedParams &p, int32_t fid, i
     }
 }
 
+// ---- the matchers' resolve step ------------------------------------------------------------------------
+
+struct Resolved {
+    int32_t fid;  // table row, -1 = miss, -2 = resolved id outside the table (zero row + status)
+    int32_t tok;  // token whose base row the position needs, or -1
+    int32_t len;  // match length (matching only)
+};
+
+// Position lane / P of tile `tile`: the given f-gram id, or the longest match over the token window `wtok`, which is
+// replaced by the window of the matcher's next tile `ntile` (requested before the dependent probe chain of this one).
+// A miss needs its base row as the fallback, and so does a hit under the additive combine (`add`).
+template <int P>
+__device__ __forceinline__ Resolved resolve_position(const EmbedParams &p, bool add, int64_t tile, int64_t ntile, int lane, int back,
+                                                     int32_t &wtok) {
+    constexpr int G = 32 / P;
+    const int64_t i = tile * G + lane / P;
+    Resolved r{-1, -1, 0};
+    if (p.fgram_in) {
+        if (i < p.T) {
+            r.fid = __ldg(p.fgram_in + i);
+            if (r.fid >= p.num_rows) r.fid = -2;  // caller error: zero row + status
+            if (r.fid == -1 || (add && r.fid >= 0)) {
+                const int64_t t64 = __ldg(p.ids + i);
+                if (t64 >= 0 && t64 < p.V) r.tok = (int32_t)t64;
+            }
+        }
+    } else {
+        int32_t ntok = -1;
+        if (ntile < p.num_tiles) ntok = load_window_token<P>(p.ids, p.T, ntile * G, lane, back);
+        const WindowMatch m = match_window<P>(p.ix, wtok, p.T, p.L, tile * G, lane, back);
+        r.fid = m.fid;
+        r.len = m.len;
+        r.tok = own_token<P>(wtok, lane, back);
+        if ((int64_t)r.tok >= p.V) r.tok = -1;
+        wtok = ntok;
+        if (r.fid != -1 && !(add && r.fid >= 0)) r.tok = -1;
+    }
+    return r;
+}
+
 // ---- the kernel --------------------------------------------------------------------------------------
 
 template <int QUANT, int OUT, int P, int U, int NM, int NG, int MINB>
@@ -240,40 +282,18 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_kernel(const Embed
         if (!p.fgram_in && tile < p.num_tiles) wtok = load_window_token<P>(p.ids, p.T, tile * G, lane, back);
         for (; tile < p.num_tiles; it += NM, tile += (int64_t)NM * gridDim.x) {
             const int q = (int)(it % R);
-            const int64_t base = tile * G;
-            const int64_t i = base + j;
-            // the ids of this warp's NEXT tile are requested before the dependent probe chain of this one
-            const int64_t ntile = tile + (int64_t)NM * gridDim.x;
-            int32_t ntok = -1;
-            int32_t fid = -1, tok = -1;
-            if (p.fgram_in) {
-                if (i < p.T) {
-                    fid = __ldg(p.fgram_in + i);
-                    if (fid >= p.num_rows) fid = -2;  // caller error: zero row + status
-                    if (fid == -1 || (p.additive && fid >= 0)) {
-                        const int64_t t64 = __ldg(p.ids + i);
-                        if (t64 >= 0 && t64 < p.V) tok = (int32_t)t64;
-                    }
-                }
-            } else {
-                if (ntile < p.num_tiles) ntok = load_window_token<P>(p.ids, p.T, ntile * G, lane, back);
-                const WindowMatch m = match_window<P>(p.ix, wtok, p.T, p.L, base, lane, back);
-                fid = m.fid;
-                tok = own_token<P>(wtok, lane, back);
-                if ((int64_t)tok >= p.V) tok = -1;
-                if ((lane % P) == 0 && i < p.T) {
-                    if (p.out_id) p.out_id[i] = m.fid;
-                    if (p.out_len) p.out_len[i] = (uint8_t)m.len;
-                }
-                wtok = ntok;
+            const int64_t i = tile * G + j;
+            const Resolved r = resolve_position<P>(p, p.additive != 0, tile, tile + (int64_t)NM * gridDim.x, lane, back, wtok);
+            if (!p.fgram_in && (lane % P) == 0 && i < p.T) {
+                if (p.out_id) p.out_id[i] = r.fid;
+                if (p.out_len) p.out_len[i] = (uint8_t)r.len;
             }
             mbar_wait(&empty_bar[q], (uint32_t)(((it / R) & 1) ^ 1));
             // lane 0 publishes the whole tile and then arrives: one producer thread per phase
-            const int32_t tk = (fid == -1 || (p.additive && fid >= 0)) ? tok : -1;  // the base row is needed
 #pragma unroll
             for (int g = 0; g < G; ++g) {
-                const int32_t f = __shfl_sync(0xFFFFFFFFu, fid, g * P);
-                const int32_t k2 = __shfl_sync(0xFFFFFFFFu, tk, g * P);
+                const int32_t f = __shfl_sync(0xFFFFFFFFu, r.fid, g * P);
+                const int32_t k2 = __shfl_sync(0xFFFFFFFFu, r.tok, g * P);
                 if (lane == 0) ring[q][g] = make_int2(f, k2);
             }
             if (lane == 0) mbar_arrive(&full_bar[q]);
@@ -320,14 +340,6 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_kernel(const Embed
 // position into the tile's ring slot; the slot's mbarrier completes when the matcher has arrived AND all row
 // bytes have landed.  Loads in flight are then bounded by shared memory (tens of KB per CTA) instead of by the
 // gather warps' registers, and the gather warps only touch shared memory and issue the output stores.
-
-struct BulkLayout {
-    int ring;        // ring slots (tiles in flight per CTA)
-    int slot_bytes;  // bytes reserved per position: the row (>= max(row_stride, 2 D)) [+ base row] [+ position row], multiple of 128
-    int pos_off;     // offset of the position-embedding row inside a position's slot, 0 = no position add
-    int add_off;     // offset of the base row staged next to a HIT's table row (additive combine), 0 = replace mode
-    int smem_bytes;  // dynamic shared memory per CTA
-};
 
 // 8 elements (chunk c) of a table row staged in shared memory -> fp32
 template <int QUANT>
@@ -399,16 +411,10 @@ __device__ __forceinline__ void stream_from_smem(const EmbedParams &p, const uin
     }
 }
 
-constexpr int kMaxRing = 16;
-// bytes of barriers + ring metadata in front of the row slots
-__host__ __device__ constexpr int bulk_header_bytes(int G) { return (2 * kMaxRing * 8 + kMaxRing * G * 8 + 127) / 128 * 128; }
-
-// ADD (compile time) = the additive combine: measured as a run-time flag it cost the plain path 1-7 % (config 1 6.56 vs
-// 6.28 us, config 2 + wpe 57.2 vs 53.1 us, config 3 1017 vs 1006 us), so the plain kernels do not carry it.
-template <int QUANT, int OUT, int P, int NM, int NG, int MINB, bool ADD>
+// The plain path only: no position rows, no additive combine (those run on embed_pipe_kernel, DESIGN section 4.2).
+template <int QUANT, int OUT, int P, int NM, int NG, int MINB>
 __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const EmbedParams p, const BulkLayout lay) {
     constexpr int G = 32 / P;
-    const int add_off = ADD ? lay.add_off : 0;
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem);
     uint64_t *empty_bar = full_bar + kMaxRing;
@@ -453,74 +459,43 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
         }
         for (; tile < p.num_tiles; it += NM, tile += (int64_t)NM * gridDim.x) {
             const int q = (int)(it % R);
-            const int64_t base = tile * G;
-            const int64_t i = base + j;
-            const int64_t ntile = tile + (int64_t)NM * gridDim.x;
-            int32_t ntok = -1;
-            int32_t fid = -1, tok = -1, mlen = 0;
-            if (p.fgram_in) {
-                if (i < p.T) {
-                    fid = __ldg(p.fgram_in + i);
-                    if (fid >= p.num_rows) fid = -2;
-                    if (fid == -1 || (ADD && fid >= 0)) {
-                        const int64_t t64 = __ldg(p.ids + i);
-                        if (t64 >= 0 && t64 < p.V) tok = (int32_t)t64;
-                    }
-                }
-            } else {
-                if (ntile < p.num_tiles) ntok = load_window_token<P>(p.ids, p.T, ntile * G, lane, back);
-                const WindowMatch m = match_window<P>(p.ix, wtok, p.T, p.L, base, lane, back);
-                fid = m.fid;
-                mlen = m.len;
-                tok = own_token<P>(wtok, lane, back);
-                if ((int64_t)tok >= p.V) tok = -1;
-                wtok = ntok;
-            }
-            if (fid != -1 && !(ADD && fid >= 0)) tok = -1;  // additive: a hit still needs its base row
+            const int64_t i = tile * G + j;
+            const Resolved r = resolve_position<P>(p, false, tile, tile + (int64_t)NM * gridDim.x, lane, back, wtok);
             // source of this position's bytes
             const bool owner = (lane % P) == 0 && i < p.T;
             const uint8_t *src = nullptr;
             uint32_t bytes = 0;
             if (owner) {
-                if (fid >= 0) {
-                    src = row_ptr(p, fid);
+                if (r.fid >= 0) {
+                    src = row_ptr(p, r.fid);
                     bytes = (uint32_t)p.row_stride;
-                } else if (tok >= 0) {
-                    src = p.base + (int64_t)tok * p.D * 2;
+                } else if (r.tok >= 0) {
+                    src = p.base + (int64_t)r.tok * p.D * 2;
                     bytes = (uint32_t)p.D * 2u;
                 }
             }
-            // additive combine: the base row of a hit rides along too (language_model.py:239-243 fused)
-            const uint8_t *src3 = nullptr;
-            if (add_off && owner && fid >= 0 && tok >= 0) src3 = p.base + (int64_t)tok * p.D * 2;
-            // the position-embedding row rides along into the same slot (language_model.py:253-254 fused)
-            const uint8_t *src2 = nullptr;
-            if (lay.pos_off && owner) src2 = p.pos + pos_in_row(i, p.L, p.T) * p.D * 2;
-            uint32_t total = bytes + (src2 ? (uint32_t)p.D * 2u : 0u) + (src3 ? (uint32_t)p.D * 2u : 0u);
+            uint32_t total = bytes;
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) total += __shfl_xor_sync(0xFFFFFFFFu, total, o);
             mbar_wait(&empty_bar[q], (uint32_t)(((it / R) & 1) ^ 1));
             // lane 0 publishes the whole tile and then arrives: one producer thread per phase
 #pragma unroll
             for (int g = 0; g < G; ++g) {
-                const int32_t f = __shfl_sync(0xFFFFFFFFu, fid, g * P);
-                const int32_t k2 = __shfl_sync(0xFFFFFFFFu, tok, g * P);
+                const int32_t f = __shfl_sync(0xFFFFFFFFu, r.fid, g * P);
+                const int32_t k2 = __shfl_sync(0xFFFFFFFFu, r.tok, g * P);
                 if (lane == 0) ring[q * G + g] = make_int2(f, k2);
             }
             if (lane == 0) mbar_arrive_expect_tx(&full_bar[q], total);
             __syncwarp();
-            uint8_t *slot = rows_smem + (size_t)(q * G + j) * lay.slot_bytes;
-            if (bytes) bulk_g2s(slot, src, bytes, &full_bar[q], pol);
-            if (src2) bulk_g2s(slot + lay.pos_off, src2, (uint32_t)p.D * 2u, &full_bar[q], policy_evict_last());
-            if (src3) bulk_g2s(slot + add_off, src3, (uint32_t)p.D * 2u, &full_bar[q], pol);
+            if (bytes) bulk_g2s(rows_smem + (size_t)(q * G + j) * lay.slot_bytes, src, bytes, &full_bar[q], pol);
             // the match result is this warp's only global write: after the previous grid (see `early` above)
             if (!waited) {
                 griddep_wait();
                 waited = true;
             }
             if (!p.fgram_in && owner) {
-                if (p.out_id) p.out_id[i] = fid;
-                if (p.out_len) p.out_len[i] = (uint8_t)mlen;
+                if (p.out_id) p.out_id[i] = r.fid;
+                if (p.out_len) p.out_len[i] = (uint8_t)r.len;
             }
         }
     } else {
@@ -541,11 +516,9 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
                 const int2 e = ring[q * G + j];
                 const int64_t t = tile * G + j;
                 if (t < p.T) {
-                    const uint8_t *slot = rows_smem + (size_t)(q * G + j) * lay.slot_bytes;
-                    const uint8_t *arow = (add_off && e.x >= 0 && e.y >= 0) ? slot + add_off : nullptr;
-                    stream_from_smem<QUANT, OUT>(p, slot, arow, lay.pos_off ? slot + lay.pos_off : nullptr, e.x, e.y, p.out + t * p.D * 2, lane,
-                                                 pol);
-                    flagged |= e.y < 0 && (e.x < 0 || add_off);
+                    stream_from_smem<QUANT, OUT>(p, rows_smem + (size_t)(q * G + j) * lay.slot_bytes, nullptr, nullptr, e.x, e.y,
+                                                 p.out + t * p.D * 2, lane, pol);
+                    flagged |= e.y < 0 && e.x < 0;
                 }
             }
             __syncwarp();
@@ -560,35 +533,25 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_bulk_kernel(const 
 #include "embed_pipe.cuh"
 namespace scone {
 
-static int num_sms() {
-    static int n = 0;
-    if (n == 0) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0)
-            n = kNumSMsB200;
-    }
-    return n;
-}
-
-// Launches kern(p[, lay]) as a persistent grid over the call's tiles of G positions: at most MINB CTAs per SM, `smem` bytes
-// of dynamic shared memory.  Kernels are launched with programmatic stream serialization (PDL): back-to-back steps overlap this kernel's launch
-// and prologue (barrier init) with the previous kernel's tail; its griddepcontrol.wait still orders everything it reads
-// or writes after the previous grid.  Same-box A/B on B200: config 1 -8 %, config 2 -1.6 %, config 3 unchanged.
-template <auto kern, int G, int MINB, typename... Layout>
-static int launch_resident(EmbedParams &p, unsigned threads, int smem, cudaStream_t stream, Layout... lay) {
+// Launches kern(p, lay...) as planned: a persistent grid over the call's tiles, programmatic stream serialization (PDL).
+// Back-to-back steps overlap this kernel's launch and prologue (barrier init) with the previous kernel's tail; its
+// griddepcontrol.wait still orders everything it reads or writes after the previous grid.  Same-box A/B on B200: config 1
+// -8 %, config 2 -1.6 %, config 3 unchanged.
+template <auto kern, typename... Layout>
+static int launch_resident(const EmbedPlan &pl, EmbedParams &p, cudaStream_t stream, Layout... lay) {
     static int configured[64] = {0};  // per device: the attribute lives in the device's context
     int dev = 0;
     SCONE_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64 || configured[dev] < smem) {
-        SCONE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        if (dev >= 0 && dev < 64) configured[dev] = smem;
+    if (dev < 0 || dev >= 64 || configured[dev] < pl.smem_bytes) {
+        SCONE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, pl.smem_bytes));
+        if (dev >= 0 && dev < 64) configured[dev] = pl.smem_bytes;
     }
-    p.num_tiles = (p.T + G - 1) / G;
-    const int64_t resident = (int64_t)num_sms() * MINB;
+    p.num_tiles = pl.num_tiles;
+    p.stagger_ns = pl.stagger_ns;
     cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)(p.num_tiles < resident ? p.num_tiles : resident));
-    cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = (size_t)smem;
+    cfg.gridDim = dim3((unsigned)pl.grid);
+    cfg.blockDim = dim3(pl.threads);
+    cfg.dynamicSmemBytes = (size_t)pl.smem_bytes;
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -599,161 +562,48 @@ static int launch_resident(EmbedParams &p, unsigned threads, int smem, cudaStrea
     return SCONE_OK;
 }
 
-template <int QUANT, int OUT, int P, int U, int NM, int NG, int MINB>
-static int launch_ldg(EmbedParams &p, cudaStream_t stream) {
-    return launch_resident<embed_kernel<QUANT, OUT, P, U, NM, NG, MINB>, 32 / P, MINB>(p, 32 * (NM + NG), 0, stream);
-}
-
-// Ring geometry for the bulk variant; returns false when rows are too wide for the budget.
-// The ring needs at least as many slots as matchers: gather warps release tiles strictly in order, so a matcher that
-// has filled tile t - NM knows every tile <= t - NM - ring is consumed; with ring >= NM that covers t - 2 ring, i.e. its
-// parity wait on slot t % ring is never more than one phase ahead.
-static bool bulk_layout(const EmbedParams &p, int G, int nm, int budget_bytes, BulkLayout &lay) {
-    int64_t slot = p.row_stride > 2ll * p.D ? p.row_stride : 2ll * p.D;
-    slot = (slot + 127) / 128 * 128;
-    lay.pos_off = lay.add_off = 0;
-    if (p.additive) {  // room for a hit's base row behind the table row
-        lay.add_off = (int)slot;
-        slot += (2ll * p.D + 127) / 128 * 128;
+template <int QUANT, int OUT, ShapeId S, int P, bool ADD>
+static int launch_shape(const EmbedPlan &pl, EmbedParams &p, cudaStream_t stream) {
+    constexpr ShapeRow s = kShapes[S];
+    if constexpr (s.family == kBulk) {
+        return launch_resident<embed_bulk_kernel<QUANT, OUT, P, s.nm, s.ng, s.minb>>(pl, p, stream, pl.bulk);
+    } else if constexpr (s.family == kPipe) {
+        static_assert(s.nl <= 32 / P, "a loader without a position");
+        return launch_resident<embed_pipe_kernel<QUANT, OUT, P, s.nm, s.nl, s.ng, s.minb, ADD>>(pl, p, stream, pl.pipe);
+    } else {
+        return launch_resident<embed_kernel<QUANT, OUT, P, 4, s.nm, s.ng, s.minb>>(pl, p, stream);  // reads p.additive
     }
-    if (p.pos) {  // room for the position-embedding row behind those
-        lay.pos_off = (int)slot;
-        slot += (2ll * p.D + 127) / 128 * 128;
-    }
-    const int64_t per_tile = slot * G;
-    int ring = (int)((budget_bytes - bulk_header_bytes(G)) / per_tile);
-    if (ring > kMaxRing) ring = kMaxRing;
-    if (ring < 2 || ring < nm) return false;
-    lay.ring = ring;
-    lay.slot_bytes = (int)slot;
-    lay.smem_bytes = bulk_header_bytes(G) + (int)(per_tile * ring);
-    return true;
 }
 
-template <int QUANT, int OUT, int P, int NM, int NG, int MINB, bool ADD>
-static int launch_bulk(EmbedParams &p, const BulkLayout &lay, cudaStream_t stream) {
-    return launch_resident<embed_bulk_kernel<QUANT, OUT, P, NM, NG, MINB, ADD>, 32 / P, MINB>(p, 32 * (NM + NG), lay.smem_bytes, stream, lay);
-}
-
-template <int QUANT, int OUT, int P, int NM, int NL, int NG, int MINB, bool ADD>
-static int launch_pipe(EmbedParams &p, const PipeLayout &lay, cudaStream_t stream) {
-    constexpr int G = 32 / P;
-    static_assert(NL <= G, "a loader without a position");
-    return launch_resident<embed_pipe_kernel<QUANT, OUT, P, NM, NL, NG, MINB, ADD>, G, MINB>(p, 32 * (NM + NL + NG), lay.smem_bytes, stream, lay);
-}
-
-// Kernel selection (measured on B200, profiles/tune_r01.md and tune_r02.md).  Rows that fit a shared-memory ring go through
-// one of the two bulk-copy kernels (embed.cu picks: single ring for the plain path, pipeline for extra rows per position and
-// for fp32 rows of 2-6 KB); the shape follows the traffic per position.  Single-ring kernel (embed_bulk_kernel):
-//   kNarrow6  < 6 KB moved, tiny rows : 6 matcher + 4 gather warps, 3 CTAs/SM, 70 KB ring  (needs >= 6 ring slots)
-//   kNarrow4  < 6 KB moved            : 4 matcher + 4 gather warps, 3 CTAs/SM, 70 KB ring  -- matcher-hungry
-//   kWide    >= 6 KB moved            : 6 matcher + 12 gather warps, 1 CTA/SM, 200 KB ring -- store-hungry
-//   kWide3   wide rows + position row : 3 matcher + 12 gather warps, 1 CTA/SM, 200 KB ring (when six slots do not fit)
-//   kWide2   wide rows + base + pos row: 2 matcher + 12 gather warps, 1 CTA/SM, 200 KB ring (two slots are enough)
-//   kMid     narrow rows + extra rows : 4 matcher + 8 gather warps, 2 CTAs/SM, 100 KB ring
-//   kSmall   anything                 : 2 matcher + 6 gather warps, 3 CTAs/SM, 70 KB ring
-//   kLdg     rows too wide for a ring : register-load variant
-// Pipeline kernel (embed_pipe_kernel; the ring only needs two full-size tiles), matcher + loader + gather warps:
-//   kNarrow6  6 + 1 + 4, 3 CTAs/SM, 70 KB    (config 2 + wpe: 47 us; + base row: 51 us)
-//   kNarrow4  5 + 2 + 4, 3 CTAs/SM, 70 KB    (plain path, fp32 rows of 3-4 KB)
-//   kMid      4 + 2 + 8, 2 CTAs/SM, 110 KB   (config 2 + base row + wpe: 56 us; fp32 rows of 5-6 KB)
-//   kWide*    6 + 4 + 12, 1 CTA/SM, 200 KB   (config 3 modes)
-//   kSmall    2 + 1 + 6, 3 CTAs/SM, 70 KB
-// A shape that does not fit with P lanes per position is retried with 2P, 4P (fewer positions per tile = smaller ring
-// slots) before the next shape is considered.
-enum Shape : int { kNarrow6 = 0, kNarrow4 = 1, kWide = 2, kSmall = 3, kLdg = 4, kWide3 = 5, kMid = 6, kWide2 = 7 };
-constexpr int kNoFit = 1;
-
-// Matcher start-up stagger (EmbedParams::stagger_ns), narrow shapes only.  Measured on config 2 (profiles/tune_r01.md):
-// 400-800 ns per matcher warp is worth 1.5 % with the pre-filter (43.3 -> 42.6 us) and 3 % without it (46.7 -> 45.3 us);
-// no effect on the wide shapes; below two tiles per matcher the delay would be exposed instead.
-template <int P, int NM, int MINB>
-static void set_stagger(EmbedParams &p) {
-    constexpr int G = 32 / P;
-    if ((p.T + G - 1) / G >= 2ll * NM * MINB * num_sms()) p.stagger_ns = 500;
-}
-
-template <int QUANT, int OUT, int P, bool ADD>
-static int launch(EmbedParams &p, cudaStream_t stream, int shape) {
-    constexpr int G = 32 / P;
-    BulkLayout lay;
-    if (p.flags & kEmbedPipe) {
-        // three-role pipeline (embed_pipe.cuh): tiles keep their full size, the row ring only needs two slots
-        PipeLayout pl;
-        switch (shape) {
-            case kNarrow6:
-                if (pipe_layout(p, G, 6, 70 * 1024, pl)) {
-                    set_stagger<P, 6, 3>(p);
-                    return launch_pipe<QUANT, OUT, P, 6, 1, 4, 3, ADD>(p, pl, stream);
-                }
-                return kNoFit;
-            case kNarrow4:  // two loaders: rows of 3-4 KB without extra rows (fp32 rows at D 768 / 1024)
-                if (pipe_layout(p, G, 5, 70 * 1024, pl)) {
-                    set_stagger<P, 5, 3>(p);
-                    return launch_pipe<QUANT, OUT, P, 5, (G >= 2 ? 2 : 1), 4, 3, ADD>(p, pl, stream);
-                }
-                return kNoFit;
-            case kMid:  // 110 KB x 2 CTAs/SM: two full-size tiles of narrow rows + base row + position row (config 2 "both": 56 us
-                        // against 70 us for the single-ring kernel and 75 us for one 200 KB CTA per SM)
-                if (pipe_layout(p, G, 4, 110 * 1024, pl)) return launch_pipe<QUANT, OUT, P, 4, (G >= 2 ? 2 : 1), 8, 2, ADD>(p, pl, stream);
-                return kNoFit;
-            case kWide:
-            case kWide3:
-            case kWide2:
-                if (pipe_layout(p, G, 6, 200 * 1024, pl)) return launch_pipe<QUANT, OUT, P, 6, (G >= 4 ? 4 : G), 12, 1, ADD>(p, pl, stream);
-                return kNoFit;
-            case kSmall:
-                if (pipe_layout(p, G, 2, 70 * 1024, pl)) return launch_pipe<QUANT, OUT, P, 2, 1, 6, 3, ADD>(p, pl, stream);
-                return kNoFit;
-            default:
-                return launch_ldg<QUANT, OUT, P, 4, 2, 6, 4>(p, stream);
+// K = (shape row, log2 P, ADD): launches the plan if it is that combination and kShapes lists it (nothing else is compiled)
+template <int QUANT, int OUT, int K>
+static bool launch_if_planned(const EmbedPlan &pl, EmbedParams &p, cudaStream_t stream, int &rc) {
+    constexpr ShapeId S = ShapeId(K / 8);
+    constexpr int P = 1 << (K / 2 % 4);
+    constexpr bool ADD = K % 2;
+    if constexpr (((ADD ? kShapes[S].add : kShapes[S].plain) & P) != 0) {
+        if (pl.row == S && pl.P == P && pl.add == ADD) {
+            rc = launch_shape<QUANT, OUT, S, P, ADD>(pl, p, stream);
+            return true;
         }
     }
-    switch (shape) {
-        case kNarrow6:
-            if (bulk_layout(p, G, 6, 70 * 1024, lay)) {
-                set_stagger<P, 6, 3>(p);
-                return launch_bulk<QUANT, OUT, P, 6, 4, 3, ADD>(p, lay, stream);
-            }
-            return kNoFit;
-        case kNarrow4:
-            if (bulk_layout(p, G, 4, 70 * 1024, lay)) {
-                set_stagger<P, 4, 3>(p);
-                return launch_bulk<QUANT, OUT, P, 4, 4, 3, ADD>(p, lay, stream);
-            }
-            return kNoFit;
-        case kWide:
-            if (bulk_layout(p, G, 6, 200 * 1024, lay)) return launch_bulk<QUANT, OUT, P, 6, 12, 1, ADD>(p, lay, stream);
-            return kNoFit;
-        case kWide3:
-            if (bulk_layout(p, G, 3, 200 * 1024, lay)) return launch_bulk<QUANT, OUT, P, 3, 12, 1, ADD>(p, lay, stream);
-            return kNoFit;
-        case kWide2:
-            if (bulk_layout(p, G, 2, 200 * 1024, lay)) return launch_bulk<QUANT, OUT, P, 2, 12, 1, ADD>(p, lay, stream);
-            return kNoFit;
-        case kMid:
-            if (bulk_layout(p, G, 4, 100 * 1024, lay)) return launch_bulk<QUANT, OUT, P, 4, 8, 2, ADD>(p, lay, stream);
-            return kNoFit;
-        case kSmall:
-            if (bulk_layout(p, G, 2, 70 * 1024, lay)) return launch_bulk<QUANT, OUT, P, 2, 6, 3, ADD>(p, lay, stream);
-            return kNoFit;
-        default:
-            return launch_ldg<QUANT, OUT, P, 4, 2, 6, 4>(p, stream);
-    }
+    return false;
 }
 
+template <int QUANT, int OUT, int... K>
+static int launch_planned(const EmbedPlan &pl, EmbedParams &p, cudaStream_t stream, std::integer_sequence<int, K...>) {
+    int rc = SCONE_OK;
+    if (!(launch_if_planned<QUANT, OUT, K>(pl, p, stream, rc) || ...)) {
+        set_error("scone_embed: no kernel compiled for shape %d, P %d, additive %d", (int)pl.row, pl.P, (int)pl.add);
+        return SCONE_E_INVALID;
+    }
+    return rc;
+}
+
+// one per (table format, output type): embed_inst.cu
 template <int QUANT, int OUT>
-static int launch_p(int P, EmbedParams &p, cudaStream_t stream, int shape) {
-    if (p.additive) {  // additive kernels exist for 4 and 8 lanes per position only (any P >= the vocabulary's is valid)
-        if (P <= 4) return launch<QUANT, OUT, 4, true>(p, stream, shape);
-        return launch<QUANT, OUT, 8, true>(p, stream, shape);
-    }
-    switch (P) {
-        case 1: return launch<QUANT, OUT, 1, false>(p, stream, shape);
-        case 2: return launch<QUANT, OUT, 2, false>(p, stream, shape);
-        case 4: return launch<QUANT, OUT, 4, false>(p, stream, shape);
-        default: return launch<QUANT, OUT, 8, false>(p, stream, shape);
-    }
+int launch_plan(const EmbedPlan &pl, EmbedParams &p, cudaStream_t stream) {
+    return launch_planned<QUANT, OUT>(pl, p, stream, std::make_integer_sequence<int, kNumShapes * 8>{});
 }
 
 }  // namespace scone

@@ -26,23 +26,8 @@
 
 namespace scone {
 
-constexpr int kMaxMetaRing = 32;
-
-struct PipeLayout {
-    int ring;        // row-ring slots (tiles staged or being consumed)
-    int meta_ring;   // metadata-ring slots, a multiple of NM
-    int slot_bytes;  // bytes reserved per position: table / fallback row [+ base row of a hit at add_off]
-    int add_off;
-    int pos_off;     // offset of the tile's block of G position rows (2 D bytes each, contiguous) from the tile's first slot, or 0
-    int tile_bytes;  // G slots + the position block
-    int smem_bytes;
-};
-
-// barriers, slot headers and the metadata ring in front of the row slots
-__host__ __device__ constexpr int pipe_header_bytes(int G) {
-    return ((2 * kMaxRing + 2 * kMaxMetaRing) * 8 + (kMaxRing + kMaxMetaRing) * G * 9 + 127) / 128 * 128;
-}
-
+// ADD (compile time) = the additive combine: measured as a run-time flag it cost the plain path 1-7 % (config 1 6.56 vs
+// 6.28 us, config 2 + wpe 57.2 vs 53.1 us, config 3 1017 vs 1006 us), so the plain kernels do not carry it.
 template <int QUANT, int OUT, int P, int NM, int NL, int NG, int MINB, bool ADD>
 __global__ void __launch_bounds__(32 * (NM + NL + NG), MINB) embed_pipe_kernel(const EmbedParams p, const PipeLayout lay) {
     constexpr int G = 32 / P;
@@ -92,36 +77,14 @@ __global__ void __launch_bounds__(32 * (NM + NL + NG), MINB) embed_pipe_kernel(c
         }
         for (; tile < p.num_tiles; it += NM, tile += (int64_t)NM * gridDim.x) {
             const int ms = (int)(it % MR);
-            const int64_t i = tile * G + lane / P;
-            const int64_t ntile = tile + (int64_t)NM * gridDim.x;
-            int32_t fid = -1, tok = -1, mlen = 0;
-            if (p.fgram_in) {
-                if (i < p.T) {
-                    fid = __ldg(p.fgram_in + i);
-                    if (fid >= p.num_rows) fid = -2;  // caller error: zero row + status
-                    if (fid == -1 || (ADD && fid >= 0)) {
-                        const int64_t t64 = __ldg(p.ids + i);
-                        if (t64 >= 0 && t64 < p.V) tok = (int32_t)t64;
-                    }
-                }
-            } else {
-                int32_t ntok = -1;
-                if (ntile < p.num_tiles) ntok = load_window_token<P>(p.ids, p.T, ntile * G, lane, back);
-                const WindowMatch m = match_window<P>(p.ix, wtok, p.T, p.L, tile * G, lane, back);
-                fid = m.fid;
-                mlen = m.len;
-                tok = own_token<P>(wtok, lane, back);
-                if ((int64_t)tok >= p.V) tok = -1;
-                wtok = ntok;
-            }
-            if (fid != -1 && !(ADD && fid >= 0)) tok = -1;  // the base row is needed by a miss, and by a hit of the additive combine
+            const Resolved r = resolve_position<P>(p, ADD, tile, tile + (int64_t)NM * gridDim.x, lane, back, wtok);
             mbar_wait(&meta_empty[ms], (uint32_t)(((it / MR) & 1) ^ 1));
             // lane 0 publishes the whole tile and then arrives: one producer thread per phase
 #pragma unroll
             for (int g = 0; g < G; ++g) {
-                const int32_t f = __shfl_sync(0xFFFFFFFFu, fid, g * P);
-                const int32_t k2 = __shfl_sync(0xFFFFFFFFu, tok, g * P);
-                const int32_t l2 = __shfl_sync(0xFFFFFFFFu, mlen, g * P);
+                const int32_t f = __shfl_sync(0xFFFFFFFFu, r.fid, g * P);
+                const int32_t k2 = __shfl_sync(0xFFFFFFFFu, r.tok, g * P);
+                const int32_t l2 = __shfl_sync(0xFFFFFFFFu, r.len, g * P);
                 if (lane == 0) {
                     meta[ms * G + g] = make_int2(f, k2);
                     meta_len[ms * G + g] = (uint8_t)l2;
@@ -230,33 +193,6 @@ __global__ void __launch_bounds__(32 * (NM + NL + NG), MINB) embed_pipe_kernel(c
         }
         if (flagged && p.status && lane == 0) atomicOr(p.status, SCONE_STATUS_TOKEN_OOR);
     }
-}
-
-// Row-ring geometry; false when not even two tiles of rows fit the budget.
-static bool pipe_layout(const EmbedParams &p, int G, int nm, int budget_bytes, PipeLayout &lay) {
-    int64_t slot = p.row_stride > 2ll * p.D ? p.row_stride : 2ll * p.D;
-    slot = (slot + 127) / 128 * 128;
-    lay.pos_off = lay.add_off = 0;
-    if (p.additive) {
-        lay.add_off = (int)slot;
-        slot += (2ll * p.D + 127) / 128 * 128;
-    }
-    int64_t per_tile = slot * G;
-    if (p.pos) {
-        lay.pos_off = (int)per_tile;
-        per_tile += (2ll * p.D * G + 127) / 128 * 128;
-    }
-    if (per_tile > (1 << 20) - 16) return false;  // an mbarrier phase counts at most 2^20 - 1 bytes
-    int ring = (int)((budget_bytes - pipe_header_bytes(G)) / per_tile);
-    if (ring > kMaxRing) ring = kMaxRing;
-    if (ring < 2) return false;
-    lay.ring = ring;
-    lay.meta_ring = kMaxMetaRing / nm * nm;  // a multiple of NM: a metadata slot is only ever filled by one matcher
-    if (lay.meta_ring > 4 * nm) lay.meta_ring = 4 * nm;
-    lay.slot_bytes = (int)slot;
-    lay.tile_bytes = (int)per_tile;
-    lay.smem_bytes = pipe_header_bytes(G) + (int)(per_tile * ring);
-    return true;
 }
 
 }  // namespace scone

@@ -22,8 +22,9 @@ DEV = "cuda"
 def index_format(request, monkeypatch):
     """Every test runs twice: with the library defaults (compact 16-byte slots whenever the tokens allow; the Bloom
     pre-filter consulted by large batches only; kernel chosen per mode), with the 32-byte slot format forced, the pre-filter
-    consulted for every batch size and the single-ring kernel (embed_bulk_kernel) for every mode, and with the second compact
-    slot format preferred and the three-role pipeline kernel (embed_pipe.cuh) for every mode."""
+    consulted for every batch size and the single-ring kernel (embed_bulk_kernel) for the plain path, and with the second
+    compact slot format preferred and the three-role pipeline kernel (embed_pipe.cuh) for the plain path.  Modes with extra
+    rows per position (position add, additive combine) take the pipeline in all three."""
     if request.param == "wide":
         monkeypatch.setenv("SCONE_INDEX_FORMAT", "wide")
         monkeypatch.setenv("SCONE_INDEX_FILTER", "always")

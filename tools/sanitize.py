@@ -10,7 +10,7 @@ from scone_b200.utils import synthetic as S  # noqa: E402
 
 cases = [("int8", 1024, 4, 300), ("int4", 512, 5, 70000), ("fp16", 128, 3, 300), ("int4", 4096, 5, 70000), ("fp16", 8192, 2, 300),
          ("int8", 16384, 3, 300), ("fp32", 768, 3, 300)]
-for pipe in ("0", "1"):                       # every mode through the single-ring kernel, then through the three-role pipeline kernel
+for pipe in ("0", "1"):                       # the plain path through the single-ring kernel, then through the three-role pipeline kernel (extra rows always take the pipeline)
   os.environ["SCONE_EMBED_PIPE"] = pipe
   for quant, D, max_n, V in cases:
       toks, lens = S.make_vocab_numpy(1500, max_n, V, seed=1, min_n=1 if max_n < 3 else 2)

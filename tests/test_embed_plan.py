@@ -5,57 +5,22 @@ the named workloads and check, over a grid of row geometries, the conditions the
 """
 
 import itertools
-import os
-import shutil
-import subprocess
 
 import pytest
 
-CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "scone_b200", "csrc")
-SMS = 148
+from plan_driver import PlanDriver
 
-DRIVER = r"""
-#include <cstdio>
-#include "embed_plan.h"
-using namespace scone;
-int main() {
-    long long D, rs, T;
-    int pos, add, res, P;
-    char env[8];
-    const char *fam[3] = {"bulk", "pipe", "ldg"};
-    while (scanf("%lld %lld %d %d %d %d %7s %lld", &D, &rs, &pos, &add, &res, &P, env, &T) == 8) {
-        const EmbedCall c{D, rs, pos != 0, add != 0, res != 0, P, env[0] == '-' ? nullptr : env, T, %SMS%};
-        const EmbedPlan pl = plan_embed(c);
-        const ShapeRow &s = kShapes[pl.row];
-        printf("%s nm %d nl %d ng %d minb %d budget %d P %d add %d", fam[s.family], s.nm, s.nl, s.ng, s.minb, s.budget, pl.P, (int)pl.add);
-        if (s.family == kBulk) printf(" ring %d slot %d", pl.bulk.ring, pl.bulk.slot_bytes);
-        if (s.family == kPipe)
-            printf(" ring %d meta %d slot %d add_off %d pos_off %d tile %d", pl.pipe.ring, pl.pipe.meta_ring, pl.pipe.slot_bytes,
-                   pl.pipe.add_off, pl.pipe.pos_off, pl.pipe.tile_bytes);
-        printf(" smem %d stagger %d grid %lld threads %u\n", pl.smem_bytes, pl.stagger_ns, (long long)pl.grid, pl.threads);
-    }
-}
-""".replace("%SMS%", str(SMS))
+SMS = 148
 
 
 @pytest.fixture(scope="module")
 def plan(tmp_path_factory):
     """plan(cases) -> one line per case; a case is (D, row_stride, pos, additive, resolved, P, SCONE_EMBED_PIPE or None, T)."""
-    cxx = shutil.which("g++")
-    if cxx is None:
+    try:
+        driver = PlanDriver.build(str(tmp_path_factory.mktemp("embed_plan")))
+    except FileNotFoundError:
         pytest.skip("no host C++ compiler")
-    d = tmp_path_factory.mktemp("embed_plan")
-    src, exe = d / "driver.cpp", d / "driver"
-    src.write_text(DRIVER)
-    subprocess.run([cxx, "-std=c++17", "-O2", "-Wall", "-Werror", "-I", CSRC, str(src), "-o", str(exe)], check=True)
-
-    def run(cases):
-        text = "".join(f"{D} {rs} {int(pos)} {int(add)} {int(res)} {P} {env or '-'} {T}\n" for D, rs, pos, add, res, P, env, T in cases)
-        out = subprocess.run([str(exe)], input=text, capture_output=True, text=True, check=True).stdout.splitlines()
-        assert len(out) == len(cases)
-        return out
-
-    return run
+    return lambda cases: driver.plan(cases, SMS)
 
 
 # (D, row_stride, position rows, additive, resolved ids, P, SCONE_EMBED_PIPE, T) -> the launch, recorded from the dispatch

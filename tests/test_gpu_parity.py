@@ -201,18 +201,21 @@ def test_lookup_all_max_n(max_n):
 
 # ---- table formats ---------------------------------------------------------------------------------------------
 
-@pytest.mark.parametrize("quant", ["fp32", "fp16", "int8", "int4"])
+@pytest.mark.parametrize("quant", ["fp32", "fp16", "int8", "int4", "int4/8", "int4/32", "int4/256"])   # int4/<group>: INT4 groups other than 128
 @pytest.mark.parametrize("D", [128, 768, 1024])
 def test_table_store_is_bit_identical_to_oracle_quantiser(quant, D):
     sb, S = _mods()
+    quant, group = quant.split("/")[0], int(quant.split("/")[1]) if "/" in quant else 128
+    if D % group:
+        pytest.skip("D must be a multiple of the INT4 group")
     rows = S.make_rows_numpy(300, D, seed=D)
     rows[3] = 0.0
     rows[5, 7] = 3.0
     rows[6] *= 1e-7            # int4: scale underflows fp16 -> scale 1
     rows[7] *= 1e4
-    tab = po.OracleTable.from_fp32(rows, quant)
+    tab = po.OracleTable.from_fp32(rows, quant, group)
     packed, stride, soff = S.pack_table_numpy(quant, tab.payload, tab.scales)
-    t = sb.CacheTable(300, D, quant)
+    t = sb.CacheTable(300, D, quant, group=group)
     assert (t.row_stride, t.scale_offset) == (stride, soff)
     perm = np.random.default_rng(0).permutation(300)
     t.store(torch.from_numpy(rows[perm]).to(DEV), torch.from_numpy(perm).to(DEV))
@@ -1023,22 +1026,24 @@ def test_projection_fold(Hf, H, k):
         assert np.array_equal(x_src[min(3, k - 1)], np.zeros(H, np.float32))
     # INT8 twice: row absmax exchanged between the CTAs of a cluster (one sweep; the default for 256 < H <= 2048; the large-k
     # shapes give every cluster several row tiles) and the two-sweep path
-    for quant in ("fp16", "fp16-pair-tile", "int8", "int8-two-sweeps", "int8-two-sweeps-pair-tile", "int4", "int4-pair-tile"):
-        if quant.startswith("int4") and H % 128:
-            continue                                # INT4 groups of 128 columns
+    for quant in ("fp16", "fp16-pair-tile", "int8", "int8-two-sweeps", "int8-two-sweeps-pair-tile", "int4", "int4-pair-tile", "int4-g32",
+                  "int4-g64-pair-tile"):
+        group = int(quant.split("-g")[1].split("-")[0]) if "-g" in quant else 128
+        if quant.startswith("int4") and H % group:
+            continue                                # INT4 groups of `group` columns
         if "two-sweeps" in quant:
             os.environ["SCONE_FOLD_XCH"] = "0"
         two_sm = "1" if quant.endswith("pair-tile") else "0"
         os.environ["SCONE_FOLD_2SM"] = two_sm
         x = xs[two_sm]                              # the fp32 product of the same tensor-core path
         quant = quant.split("-")[0]
-        tq = sb.CacheTable(k, H, quant)
+        tq = sb.CacheTable(k, H, quant, group=group)
         try:
             tq.store_projected(torch.from_numpy(rows).to(DEV), torch.from_numpy(W).to(DEV), row_ids=torch.from_numpy(perm).to(DEV))
         finally:
             os.environ.pop("SCONE_FOLD_XCH", None)
             os.environ.pop("SCONE_FOLD_2SM", None)
-        ref = sb.CacheTable(k, H, quant)
+        ref = sb.CacheTable(k, H, quant, group=group)
         ref.store(torch.from_numpy(x).to(DEV))
         assert torch.equal(tq.storage, ref.storage), quant
         dq = tq.gather(torch.arange(k, device=DEV)).cpu().numpy()[perm]
@@ -1047,8 +1052,13 @@ def test_projection_fold(Hf, H, k):
         elif quant == "int8":
             step = (np.abs(P).max(axis=1, keepdims=True) / 127.0) * np.ones_like(P)
         else:
-            step = np.repeat((np.abs(P).reshape(k, H // 128, 128).max(axis=2) / 7.0).astype(np.float16).astype(np.float32), 128, axis=1)
-        assert np.all(np.abs(dq - P) <= 0.51 * step + 4 * bound + 1e-30), quant
+            step = np.repeat((np.abs(P).reshape(k, H // group, group).max(axis=2) / 7.0).astype(np.float16).astype(np.float32), group, axis=1)
+        assert np.all(np.abs(dq - P) <= 0.51 * step + 4 * bound + 1e-30), (quant, group)
+    # the epilogue's per-group loop takes 32, 64 or 128 columns
+    for group in (16, 256):
+        if H % group == 0:
+            with pytest.raises(ValueError, match="group"):
+                sb.CacheTable(k, H, "int4", group=group).store_projected(torch.from_numpy(rows).to(DEV), torch.from_numpy(W).to(DEV))
     # the drop-in entry: cache_embeddings(..., projection=W) then lookup serves the projected rows
     if k < 200:
         return

@@ -384,6 +384,20 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
 }
 
 // ---------------------------------------------------------------------------------------------
+// scales of the stored formats: store_kernel and the projection fold's epilogue (held bit-identical to it) both use these
+// ---------------------------------------------------------------------------------------------
+// INT8: one fp32 scale per row, amax / 127; 1 for an all-zero row
+__device__ __forceinline__ float int8_row_scale(float amax) {
+    const float s = __fdiv_rn(amax, 127.0f);
+    return s == 0.0f ? 1.0f : s;
+}
+// INT4: one fp16 scale per group, amax / 7 (at most the fp16 maximum); 1 for an all-zero group
+__device__ __forceinline__ __half int4_group_scale(float amax) {
+    const __half s = __float2half_rn(fminf(__fdiv_rn(amax, 7.0f), 65504.0f));
+    return __half2float(s) == 0.0f ? __float2half_rn(1.0f) : s;
+}
+
+// ---------------------------------------------------------------------------------------------
 // decode of 8 consecutive elements to fp32 (exact integer -> float, then ONE fp32 multiply).
 // Values travel as four float2 pairs (elements 2k, 2k+1) so that the adds and multiplies issue as the sm_100 packed
 // instructions FADD2 / FMUL2 (two IEEE round-to-nearest fp32 operations per instruction -- the same roundings as the

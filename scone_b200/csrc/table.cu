@@ -69,8 +69,7 @@ __global__ void __launch_bounds__(256) store_kernel(uint8_t *rows, int64_t row_s
         float amax = 0.0f;
         for (int d = lane; d < D; d += 32) amax = fmaxf(amax, fabsf(x[d]));
         amax = warp_max(amax);
-        float s = __fdiv_rn(amax, 127.0f);
-        if (s == 0.0f) s = 1.0f;
+        const float s = int8_row_scale(amax);
         for (int d = lane * 4; d < D; d += 128) {
             const float4 v = *reinterpret_cast<const float4 *>(x + d);
             const float q[4] = {v.x, v.y, v.z, v.w};
@@ -93,9 +92,7 @@ __global__ void __launch_bounds__(256) store_kernel(uint8_t *rows, int64_t row_s
             float amax = 0.0f;
             for (int d = lane; d < group; d += 32) amax = fmaxf(amax, fabsf(xg[d]));
             amax = warp_max(amax);
-            float s32 = fminf(__fdiv_rn(amax, 7.0f), 65504.0f);
-            __half s16 = __float2half_rn(s32);
-            if (__half2float(s16) == 0.0f) s16 = __float2half_rn(1.0f);
+            const __half s16 = int4_group_scale(amax);
             const float sw = __half2float(s16);
             for (int d = lane * 2; d < group; d += 64) {
                 float a = fminf(fmaxf(rintf(__fdiv_rn(xg[d], sw)), -7.0f), 7.0f);

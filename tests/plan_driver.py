@@ -1,7 +1,8 @@
-"""Host-side driver of the fused path's launch plan (scone_b200/csrc/embed_plan.h), compiled with g++.
+"""Host-side driver of the launch plans of the fused path (scone_b200/csrc/embed_plan.h) and of the projection fold
+(fold_plan.h), compiled with g++.
 
-The plan is plain C++ with no CUDA header, so it runs on any host.  Tests use it to pin the kernel a call gets
-(test_embed_plan.py) and to pick, for every kernel the library compiles, a call that launches it
+The plans are plain C++ with no CUDA header, so they run on any host.  Tests use the driver to pin the kernel a call gets
+(test_embed_plan.py, test_fold_plan.py) and to pick, for every kernel the library compiles, a call that launches it
 (test_gpu_kernel_matrix.py).  A helper module, not a conftest: importing it does nothing until ``PlanDriver`` is built.
 """
 
@@ -16,14 +17,31 @@ from typing import Iterable, List, Optional, Sequence, Tuple
 CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "scone_b200", "csrc")
 FAMILIES = ("bulk", "pipe", "ldg")
 
-# argv: shapes | plan <sms> | detail <sms>.  plan / detail read one call per line:
+# argv: shapes | plan <sms> | detail <sms> | fold <sms>.  plan / detail read one call per line:
 # D row_stride pos additive resolved P SCONE_EMBED_PIPE(or -) T
+# and fold reads: quant H K k SCONE_FOLD_2SM(or -) SCONE_FOLD_XCH(or -) resident_exchange_clusters
 SOURCE = r"""
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include "embed_plan.h"
+#include "fold_plan.h"
 using namespace scone;
+static int fold(int sms) {
+    const char *path[kNumFoldPaths] = {"single", "pairs", "pairtile", "exchange"};
+    int quant, H, K, resident;
+    long long k;
+    char sm2[8], xch[8];
+    while (scanf("%d %d %d %lld %7s %7s %d", &quant, &H, &K, &k, sm2, xch, &resident) == 7) {
+        const FoldCall c{quant, H, K, k, sms, sm2[0] == '-' ? nullptr : sm2, xch[0] == '-' ? nullptr : xch, resident};
+        const FoldPlan pl = plan_fold(c);
+        const FoldPathRow &r = kFoldPaths[pl.path];
+        printf("%s cluster %d tiles %d epi %d stages %d stage_bytes %d box %d n_chunks %d k_blocks %d m_groups %d sweeps %d grid %d "
+               "threads %d\n", path[pl.path], pl.cluster, r.tiles, r.epi_warps, r.stages, r.stage_bytes, r.w_box_rows, pl.n_chunks,
+               pl.k_blocks, pl.m_groups, pl.sweeps, pl.grid, pl.threads);
+    }
+    return 0;
+}
 int main(int argc, char **argv) {
     const char *fam[3] = {"bulk", "pipe", "ldg"};
     if (argc == 2 && !strcmp(argv[1], "shapes")) {
@@ -34,6 +52,7 @@ int main(int argc, char **argv) {
         return 0;
     }
     if (argc != 3) return 2;
+    if (!strcmp(argv[1], "fold")) return fold(atoi(argv[2]));
     const bool detail = !strcmp(argv[1], "detail");
     const int sms = atoi(argv[2]);
     long long D, rs, T;
@@ -62,6 +81,8 @@ int main(int argc, char **argv) {
 
 # (D, row_stride, position rows, additive, resolved ids, P, SCONE_EMBED_PIPE or None, T)
 Call = Tuple[int, int, int, int, int, int, Optional[str], int]
+# (quant, H, K, k, SCONE_FOLD_2SM or None, SCONE_FOLD_XCH or None, resident exchange clusters)
+FoldCall = Tuple[int, int, int, int, Optional[str], Optional[str], int]
 
 
 class ShapeRow:
@@ -109,9 +130,12 @@ class PlanDriver:
 
     def _run(self, args: Sequence[str], cases: Iterable[Call]) -> List[str]:
         cases = list(cases)
-        text = "".join(f"{D} {rs} {int(pos)} {int(add)} {int(res)} {P} {env or '-'} {T}\n" for D, rs, pos, add, res, P, env, T in cases)
+        return self._lines(args, "".join(f"{D} {rs} {int(pos)} {int(add)} {int(res)} {P} {env or '-'} {T}\n"
+                                         for D, rs, pos, add, res, P, env, T in cases), len(cases))
+
+    def _lines(self, args: Sequence[str], text: str, n: int) -> List[str]:
         out = subprocess.run([self.exe, *args], input=text, capture_output=True, text=True, check=True).stdout.splitlines()
-        assert len(out) == len(cases)
+        assert len(out) == n
         return out
 
     def shapes(self) -> List[ShapeRow]:
@@ -124,3 +148,9 @@ class PlanDriver:
 
     def detail(self, cases: Iterable[Call], sms: int) -> List[Planned]:
         return [Planned(line) for line in self._run(["detail", str(sms)], cases)]
+
+    def fold(self, cases: Iterable[FoldCall], sms: int) -> List[str]:
+        """plan_fold() of each call: one line with the path, its row of kFoldPaths and the launch."""
+        cases = list(cases)
+        return self._lines(["fold", str(sms)], "".join(f"{q} {H} {K} {k} {s or '-'} {x or '-'} {res}\n" for q, H, K, k, s, x, res in cases),
+                           len(cases))

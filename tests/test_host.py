@@ -251,6 +251,10 @@ def test_c_abi_rejects_bad_arguments_without_a_gpu():
     assert b"flag" in L.scone_last_error()
     desc = _lib.TableDesc(16, 100, 4, 1, 1024, 128, 1024)                                         # row_stride 100: not a multiple of 16
     assert L.scone_table_gather(C.byref(desc), None, 1, None, 2, None, None) == _lib.E_INVALID
+    # the projection fold's TMA row coordinates are 32-bit: k = 2^31 source rows is refused (aligned stand-in pointers, never read)
+    desc = _lib.TableDesc(256, 1056, 4, 1, 1024, 128, 1024)
+    assert L.scone_table_store_projected(C.byref(desc), 512, 768, 64, 1024, 0, 1 << 31, None, None) == _lib.E_INVALID
+    assert b"k too large" in L.scone_last_error()
 
 
 def test_bench_reference_arm_runs_on_cpu():

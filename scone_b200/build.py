@@ -20,7 +20,7 @@ SOURCES = ["api.cu", "index.cu", "table.cu", "embed.cu", "pipeline.cu", "fold.cu
 # the fused path's kernels are compiled once per (table format, output type): eight translation units, in parallel
 INST_SOURCE = "embed_inst.cu"
 INSTANCES = [(q, o) for o in (0, 1) for q in (0, 1, 2, 3)]
-HEADERS = ["common.cuh", "match.cuh", "embed_plan.h", "fold_plan.h", "embed_kernels.cuh", "embed_pipe.cuh", os.path.join("..", "..", "include", "scone_b200.h")]
+HEADERS = ["common.cuh", "match.cuh", "embed_plan.h", "fold_plan.h", "row_format.cuh", "embed_kernels.cuh", "embed_pipe.cuh", os.path.join("..", "..", "include", "scone_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

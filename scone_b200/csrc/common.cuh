@@ -383,100 +383,6 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
                  : "memory");
 }
 
-// ---------------------------------------------------------------------------------------------
-// scales of the stored formats: store_kernel and the projection fold's epilogue (held bit-identical to it) both use these
-// ---------------------------------------------------------------------------------------------
-// INT8: one fp32 scale per row, amax / 127; 1 for an all-zero row
-__device__ __forceinline__ float int8_row_scale(float amax) {
-    const float s = __fdiv_rn(amax, 127.0f);
-    return s == 0.0f ? 1.0f : s;
-}
-// INT4: one fp16 scale per group, amax / 7 (at most the fp16 maximum); 1 for an all-zero group
-__device__ __forceinline__ __half int4_group_scale(float amax) {
-    const __half s = __float2half_rn(fminf(__fdiv_rn(amax, 7.0f), 65504.0f));
-    return __half2float(s) == 0.0f ? __float2half_rn(1.0f) : s;
-}
-
-// ---------------------------------------------------------------------------------------------
-// decode of 8 consecutive elements to fp32 (exact integer -> float, then ONE fp32 multiply).
-// Values travel as four float2 pairs (elements 2k, 2k+1) so that the adds and multiplies issue as the sm_100 packed
-// instructions FADD2 / FMUL2 (two IEEE round-to-nearest fp32 operations per instruction -- the same roundings as the
-// scalar forms, half the issue slots) and the pairs feed cvt.rn.{bf16x2,f16x2}.f32 directly.
-// ---------------------------------------------------------------------------------------------
-typedef float2 f32x8[4];
-
-__device__ __forceinline__ void decode_fp16x8(uint4 raw, f32x8 &x) {
-    const __half2 *h = reinterpret_cast<const __half2 *>(&raw);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) x[k] = __half22float2(h[k]);
-}
-__device__ __forceinline__ void decode_bf16x8(uint4 raw, f32x8 &x) {
-    const uint32_t *u = reinterpret_cast<const uint32_t *>(&raw);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) x[k] = make_float2(__uint_as_float(u[k] << 16), __uint_as_float(u[k] & 0xFFFF0000u));
-}
-// unquantised rows (SCONE_QUANT_FP32): eight floats = two 16-byte vectors
-__device__ __forceinline__ void decode_fp32x8(uint4 a, uint4 b, f32x8 &x) {
-    x[0] = make_float2(__uint_as_float(a.x), __uint_as_float(a.y));
-    x[1] = make_float2(__uint_as_float(a.z), __uint_as_float(a.w));
-    x[2] = make_float2(__uint_as_float(b.x), __uint_as_float(b.y));
-    x[3] = make_float2(__uint_as_float(b.z), __uint_as_float(b.w));
-}
-// int8 -> fp32 without the I2F pipe: place (q ^ 0x80) in the low mantissa byte of 2^23 and
-// subtract 2^23 + 128; both steps are exact.
-__device__ __forceinline__ void decode_int8x8(uint2 raw, float scale, f32x8 &x) {
-    const uint32_t w[2] = {raw.x ^ 0x80808080u, raw.y ^ 0x80808080u};
-    const float2 bias = make_float2(-8388736.0f, -8388736.0f), sc = make_float2(scale, scale);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const uint32_t m0 = __byte_perm(w[k >> 1], 0x4B000000u, 0x7650 + ((2 * k) & 3));  // bytes: [q, 0, 0, 0x4B]
-        const uint32_t m1 = __byte_perm(w[k >> 1], 0x4B000000u, 0x7650 + ((2 * k + 1) & 3));
-        x[k] = __fmul2_rn(__fadd2_rn(make_float2(__uint_as_float(m0), __uint_as_float(m1)), bias), sc);
-    }
-}
-// eight nibbles (q + 8), element 0 in the lowest nibble: split into even / odd elements (one byte each), then the
-// same mantissa placement as int8
-__device__ __forceinline__ void decode_int4x8(uint32_t raw, float scale, f32x8 &x) {
-    const uint32_t ev = raw & 0x0F0F0F0Fu, od = (raw >> 4) & 0x0F0F0F0Fu;  // elements 0,2,4,6 / 1,3,5,7
-    const float2 bias = make_float2(-8388616.0f, -8388616.0f), sc = make_float2(scale, scale);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const uint32_t m0 = __byte_perm(ev, 0x4B000000u, 0x7650 + k);
-        const uint32_t m1 = __byte_perm(od, 0x4B000000u, 0x7650 + k);
-        x[k] = __fmul2_rn(__fadd2_rn(make_float2(__uint_as_float(m0), __uint_as_float(m1)), bias), sc);
-    }
-}
-__device__ __forceinline__ void zero8(f32x8 &x) {
-#pragma unroll
-    for (int k = 0; k < 4; ++k) x[k] = make_float2(0.0f, 0.0f);
-}
-// x += y, eight fp32 round-to-nearest adds (four FADD2)
-__device__ __forceinline__ void add8(f32x8 &x, const f32x8 &y) {
-#pragma unroll
-    for (int k = 0; k < 4; ++k) x[k] = __fadd2_rn(x[k], y[k]);
-}
-
-__device__ __forceinline__ uint4 pack_bf16x8(const f32x8 &x) {
-    uint4 r;
-    uint32_t *u = reinterpret_cast<uint32_t *>(&r);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        __nv_bfloat162 b = __float22bfloat162_rn(x[k]);
-        u[k] = *reinterpret_cast<uint32_t *>(&b);
-    }
-    return r;
-}
-__device__ __forceinline__ uint4 pack_fp16x8(const f32x8 &x) {
-    uint4 r;
-    uint32_t *u = reinterpret_cast<uint32_t *>(&r);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        __half2 b = __float22half2_rn(x[k]);
-        u[k] = *reinterpret_cast<uint32_t *>(&b);
-    }
-    return r;
-}
-
 #endif  // __CUDACC__
 
 }  // namespace scone

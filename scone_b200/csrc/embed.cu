@@ -42,8 +42,6 @@ static int dispatch(int P, bool resolved, EmbedParams &p, int quant, int out_dty
     return SCONE_OK;
 }
 
-int check_table(const scone_table_desc_t *t, const char *who);  // table.cu
-
 static int fill_table(EmbedParams &p, const scone_table_desc_t *t, const char *who) {
     int rc = check_table(t, who);
     if (rc != SCONE_OK) return rc;
@@ -54,12 +52,7 @@ static int fill_table(EmbedParams &p, const scone_table_desc_t *t, const char *w
     p.num_rows = t->num_rows;
     p.D = t->dim;
     p.scale_off = t->scale_offset;
-    p.group_shift = 0;
-    if (t->quant == SCONE_QUANT_INT4) {
-        int g8 = t->group / 8, sh = 0;
-        while ((1 << sh) < g8) ++sh;
-        p.group_shift = sh;
-    }
+    p.group_shift = group_shift(t->group);
     return SCONE_OK;
 }
 

@@ -26,9 +26,9 @@
 //
 // This header is compiled once per (table format, output type) by embed_inst.cu; embed.cu holds the plan and the C ABI.
 #pragma once
-#include "common.cuh"
 #include "embed_plan.h"
 #include "match.cuh"
+#include "row_format.cuh"
 
 #include <utility>
 
@@ -60,12 +60,6 @@ struct EmbedParams {
     uint32_t flags;       // SCONE_EMBED_* of scone_embed_opts_t
 };
 
-// row bytes holding 8 consecutive elements of a stored row
-template <int QUANT>
-__host__ __device__ constexpr int chunk_bytes() {
-    return QUANT == SCONE_QUANT_FP32 ? 32 : QUANT == SCONE_QUANT_FP16 ? 16 : QUANT == SCONE_QUANT_INT8 ? 8 : 4;
-}
-
 // address of table row `fid`: local, or on the peer that owns it (NVLink)
 __device__ __forceinline__ const uint8_t *row_ptr(const EmbedParams &p, int32_t fid) {
     if (p.world == 1) return p.rows + (int64_t)fid * p.row_stride;
@@ -80,63 +74,65 @@ constexpr int kRing = 16;  // tiles embed_kernel's matchers may run ahead of the
 // programmatic dependent launch: block until the grid this one was launched behind has completed and its writes are visible
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
+// base and position rows are stored in the output type
 template <int OUT>
 __device__ __forceinline__ void decode16x8(uint4 raw, f32x8 &x) {
     if (OUT == SCONE_OUT_BF16) decode_bf16x8(raw, x);
     else decode_fp16x8(raw, x);
 }
-template <int OUT>
-__device__ __forceinline__ uint4 pack16x8(const f32x8 &x) {
-    return OUT == SCONE_OUT_BF16 ? pack_bf16x8(x) : pack_fp16x8(x);
-}
 
 // ---- streaming one position -------------------------------------------------------------------------
+
+// A table row's chunk in the output type.  FP16 rows into FP16 output are copied as they are.
+template <int QUANT, int OUT>
+__device__ __forceinline__ uint4 hit_chunk(const RawChunk &raw) {
+    if (QUANT == SCONE_QUANT_FP16 && OUT == SCONE_OUT_FP16) return raw.a;
+    f32x8 x;
+    decode_chunk<QUANT>(raw, x);
+    return pack_chunk<OUT>(x).v[0];
+}
+
+// Chunk c of a position that needs more than its table row, in fp32 (the caller packs it to the output type): the table
+// row (fid >= 0) or else the fallback row (tok >= 0), both at `src`, or else zeros; + the base row `arow` (additive combine:
+// wte(ids) + f-gram row); + the position row `prow`.  The one statement of these fp32 adds and their order for every kernel:
+// the output is held bit-exact to the oracle.  Position rows are read through `pmem`.
+template <int QUANT, int OUT, class Mem, class PosMem>
+__device__ __forceinline__ void combine_chunk(const EmbedParams &p, const Mem &mem, const PosMem &pmem, int32_t fid, int32_t tok,
+                                              const uint8_t *src, float rs, const uint8_t *arow, const uint8_t *prow, int c, f32x8 &x) {
+    if (fid >= 0) decode_chunk<QUANT>(load_chunk<QUANT>(mem, src, c, p.scale_off, p.group_shift, rs), x);
+    else if (tok >= 0) decode16x8<OUT>(mem.v16(src + c * 16), x);
+    else zero8(x);
+    if (arow) {
+        f32x8 y;
+        decode16x8<OUT>(mem.v16(arow + c * 16), y);
+        add8(x, y);
+    }
+    if (prow) {
+        f32x8 y;
+        decode16x8<OUT>(pmem.v16(prow + c * 16), y);
+        add8(x, y);
+    }
+}
 
 // Hit: dequantise table row `fid` into dst.  U 256-element steps in flight per lane.
 template <int QUANT, int OUT, int U>
 __device__ __forceinline__ void stream_hit(const EmbedParams &p, int32_t fid, uint8_t *__restrict__ dst, int lane, uint64_t pol) {
     const uint8_t *__restrict__ row = row_ptr(p, fid);
     const int nchunks = p.D >> 3;
-    float rs = 1.0f;
-    if (QUANT == SCONE_QUANT_INT8) rs = __ldg(reinterpret_cast<const float *>(row + p.scale_off));
+    const GlobalRowsEvictFirst mem{{}, pol};
+    const float rs = row_scale<QUANT>(mem, row, p.scale_off);
     for (int c0 = lane; c0 < nchunks; c0 += 32 * U) {
-        uint4 raw[U], rawb[U];  // rawb: second half of an fp32 chunk
-        float sc[U];
+        RawChunk raw[U];
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             const int c = c0 + 32 * u;
-            sc[u] = rs;
-            if (c < nchunks) {
-                if (QUANT == SCONE_QUANT_FP32) {
-                    raw[u] = ldg_stream_16(row + c * 32, pol);
-                    rawb[u] = ldg_stream_16(row + c * 32 + 16, pol);
-                } else if (QUANT == SCONE_QUANT_FP16) {
-                    raw[u] = ldg_stream_16(row + c * 16, pol);
-                } else if (QUANT == SCONE_QUANT_INT8) {
-                    const uint2 v = ldg_stream_8(row + c * 8, pol);
-                    raw[u].x = v.x;
-                    raw[u].y = v.y;
-                } else {
-                    raw[u].x = ldg_stream_4(row + c * 4, pol);
-                    sc[u] = __half2float(__ldg(reinterpret_cast<const __half *>(row + p.scale_off) + (c >> p.group_shift)));
-                }
-            }
+            if (c < nchunks) raw[u] = load_chunk<QUANT>(mem, row, c, p.scale_off, p.group_shift, rs);
         }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             const int c = c0 + 32 * u;
             if (c < nchunks) {
-                uint4 o;
-                if (QUANT == SCONE_QUANT_FP16 && OUT == SCONE_OUT_FP16) {
-                    o = raw[u];
-                } else {
-                    f32x8 x;
-                    if (QUANT == SCONE_QUANT_FP32) decode_fp32x8(raw[u], rawb[u], x);
-                    else if (QUANT == SCONE_QUANT_FP16) decode_fp16x8(raw[u], x);
-                    else if (QUANT == SCONE_QUANT_INT8) decode_int8x8(make_uint2(raw[u].x, raw[u].y), sc[u], x);
-                    else decode_int4x8(raw[u].x, sc[u], x);
-                    o = pack16x8<OUT>(x);
-                }
+                const uint4 o = hit_chunk<QUANT, OUT>(raw[u]);
                 stg_stream_16(dst + c * 16, o, pol);
             }
         }
@@ -168,39 +164,15 @@ template <int QUANT, int OUT>
 __device__ __noinline__ void stream_general(const EmbedParams &p, int32_t fid, int32_t tok, int64_t t, uint8_t *__restrict__ dst,
                                             int lane) {
     const int nchunks = p.D >> 3;
-    const uint8_t *row = fid >= 0 ? row_ptr(p, fid) : nullptr;
-    const uint8_t *brow = (fid < 0 && tok >= 0) ? p.base + (int64_t)tok * p.D * 2 : nullptr;
+    const GlobalRows mem;
+    const uint8_t *src = fid >= 0 ? row_ptr(p, fid) : tok >= 0 ? p.base + (int64_t)tok * p.D * 2 : nullptr;
+    const float rs = fid >= 0 ? row_scale<QUANT>(mem, src, p.scale_off) : 1.0f;
     const uint8_t *arow = (p.additive && fid >= 0 && tok >= 0) ? p.base + (int64_t)tok * p.D * 2 : nullptr;
     const uint8_t *prow = p.pos ? p.pos + pos_in_row(t, p.L, p.T) * p.D * 2 : nullptr;
     for (int c = lane; c < nchunks; c += 32) {
         f32x8 x;
-        if (row) {
-            if (QUANT == SCONE_QUANT_FP32) {
-                decode_fp32x8(ldg_stream_16(row + c * 32), ldg_stream_16(row + c * 32 + 16), x);
-            } else if (QUANT == SCONE_QUANT_FP16) {
-                decode_fp16x8(ldg_stream_16(row + c * 16), x);
-            } else if (QUANT == SCONE_QUANT_INT8) {
-                decode_int8x8(ldg_stream_8(row + c * 8), __ldg(reinterpret_cast<const float *>(row + p.scale_off)), x);
-            } else {
-                const __half hs = __ldg(reinterpret_cast<const __half *>(row + p.scale_off) + (c >> p.group_shift));
-                decode_int4x8(ldg_stream_4(row + c * 4), __half2float(hs), x);
-            }
-        } else if (brow) {
-            decode16x8<OUT>(ldg_stream_16(brow + c * 16), x);
-        } else {
-            zero8(x);
-        }
-        if (arow) {  // wte(ids) + f-gram row
-            f32x8 y;
-            decode16x8<OUT>(ldg_stream_16(arow + c * 16), y);
-            add8(x, y);
-        }
-        if (prow) {
-            f32x8 y;
-            decode16x8<OUT>(__ldg(reinterpret_cast<const uint4 *>(prow + c * 16)), y);
-            add8(x, y);
-        }
-        stg_stream_16(dst + c * 16, pack16x8<OUT>(x));
+        combine_chunk<QUANT, OUT>(p, mem, GlobalRowsCached{}, fid, tok, src, rs, arow, prow, c, x);
+        stg_stream_16(dst + c * 16, pack_chunk<OUT>(x).v[0]);
     }
 }
 
@@ -341,38 +313,16 @@ __global__ void __launch_bounds__(32 * (NM + NG), MINB) embed_kernel(const Embed
 // bytes have landed.  Loads in flight are then bounded by shared memory (tens of KB per CTA) instead of by the
 // gather warps' registers, and the gather warps only touch shared memory and issue the output stores.
 
-// 8 elements (chunk c) of a table row staged in shared memory -> fp32
-template <int QUANT>
-__device__ __forceinline__ void decode_smem(const EmbedParams &p, const uint8_t *srow, int c, float rs, f32x8 &x) {
-    if (QUANT == SCONE_QUANT_FP32) {
-        decode_fp32x8(*reinterpret_cast<const uint4 *>(srow + c * 32), *reinterpret_cast<const uint4 *>(srow + c * 32 + 16), x);
-    } else if (QUANT == SCONE_QUANT_FP16) {
-        decode_fp16x8(*reinterpret_cast<const uint4 *>(srow + c * 16), x);
-    } else if (QUANT == SCONE_QUANT_INT8) {
-        decode_int8x8(*reinterpret_cast<const uint2 *>(srow + c * 8), rs, x);
-    } else {
-        const float sc = __half2float(*(reinterpret_cast<const __half *>(srow + p.scale_off) + (c >> p.group_shift)));
-        decode_int4x8(*reinterpret_cast<const uint32_t *>(srow + c * 4), sc, x);
-    }
-}
-
 template <int QUANT, int OUT>
 __device__ __forceinline__ void stream_from_smem(const EmbedParams &p, const uint8_t *srow, const uint8_t *arow, const uint8_t *prow,
                                                  int32_t fid, int32_t tok, uint8_t *__restrict__ dst, int lane, uint64_t pol) {
     const int nchunks = p.D >> 3;  // arow / prow: base row to add to a hit / position-embedding row, in shared memory, or NULL
+    const SharedRows mem;
     if (fid >= 0 && !prow && !arow) {
-        float rs = 1.0f;
-        if (QUANT == SCONE_QUANT_INT8) rs = *reinterpret_cast<const float *>(srow + p.scale_off);
+        const float rs = row_scale<QUANT>(mem, srow, p.scale_off);
 #pragma unroll 4
         for (int c = lane; c < nchunks; c += 32) {
-            uint4 o;
-            if (QUANT == SCONE_QUANT_FP16 && OUT == SCONE_OUT_FP16) {
-                o = *reinterpret_cast<const uint4 *>(srow + c * 16);
-            } else {
-                f32x8 x;
-                decode_smem<QUANT>(p, srow, c, rs, x);
-                o = pack16x8<OUT>(x);
-            }
+            const uint4 o = hit_chunk<QUANT, OUT>(load_chunk<QUANT>(mem, srow, c, p.scale_off, p.group_shift, rs));
             stg_stream_16(dst + c * 16, o, pol);
         }
     } else if (fid < 0 && tok >= 0 && !prow) {
@@ -381,31 +331,15 @@ __device__ __forceinline__ void stream_from_smem(const EmbedParams &p, const uin
     } else {
         // base-row add, position add (the matcher staged those rows next to the table row) / zero row
         float rs = 1.0f;
-        if (QUANT == SCONE_QUANT_INT8 && fid >= 0) rs = *reinterpret_cast<const float *>(srow + p.scale_off);
+        if (fid >= 0) rs = row_scale<QUANT>(mem, srow, p.scale_off);
         for (int c0 = lane; c0 < nchunks; c0 += 128) {
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 const int c = c0 + 32 * u;
                 if (c >= nchunks) continue;
                 f32x8 x;
-                if (fid >= 0) {
-                    decode_smem<QUANT>(p, srow, c, rs, x);
-                } else if (tok >= 0) {
-                    decode16x8<OUT>(*reinterpret_cast<const uint4 *>(srow + c * 16), x);
-                } else {
-                    zero8(x);
-                }
-                if (arow) {  // wte(ids) + f-gram row
-                    f32x8 y;
-                    decode16x8<OUT>(*reinterpret_cast<const uint4 *>(arow + c * 16), y);
-                    add8(x, y);
-                }
-                if (prow) {
-                    f32x8 y;
-                    decode16x8<OUT>(*reinterpret_cast<const uint4 *>(prow + c * 16), y);
-                    add8(x, y);
-                }
-                stg_stream_16(dst + c * 16, pack16x8<OUT>(x), pol);
+                combine_chunk<QUANT, OUT>(p, mem, mem, fid, tok, srow, rs, arow, prow, c, x);
+                stg_stream_16(dst + c * 16, pack_chunk<OUT>(x).v[0], pol);
             }
         }
     }

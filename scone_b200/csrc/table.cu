@@ -4,7 +4,7 @@
 // get_embeddings gather (:113-147).  The reference keeps fp32 rows; the three stored formats and
 // their formulas are defined in oracle/py_oracle.py (SURVEY.md section 8c) and implemented here
 // with the same fp32 operations in the same order, so the stored bits are identical.
-#include "common.cuh"
+#include "row_format.cuh"
 
 namespace scone {
 
@@ -16,21 +16,15 @@ int check_table(const scone_table_desc_t *t, const char *who) {
     SCONE_REQUIRE(t->row_stride > 0 && t->row_stride % 16 == 0, "%s: row_stride %lld must be a positive multiple of 16", who,
                   (long long)t->row_stride);
     SCONE_REQUIRE(((uintptr_t)t->d_rows & 15) == 0, "%s: table rows pointer must be 16-byte aligned", who);
-    int64_t need = 0;
-    if (t->quant == SCONE_QUANT_FP32) {
-        need = 4ll * t->dim;
-    } else if (t->quant == SCONE_QUANT_FP16) {
-        need = 2ll * t->dim;
-    } else if (t->quant == SCONE_QUANT_INT8) {
-        SCONE_REQUIRE(t->scale_offset >= t->dim && t->scale_offset % 4 == 0, "%s: INT8 scale_offset %d invalid", who, t->scale_offset);
-        need = t->scale_offset + 4ll;
-    } else {
-        const int g = t->group;
-        SCONE_REQUIRE(g >= 8 && (g & (g - 1)) == 0, "%s: INT4 group %d must be a power of two >= 8", who, g);
-        SCONE_REQUIRE(t->dim % g == 0, "%s: dim %d not a multiple of group %d", who, t->dim, g);
-        SCONE_REQUIRE(t->scale_offset >= t->dim / 2 && t->scale_offset % 2 == 0, "%s: INT4 scale_offset %d invalid", who, t->scale_offset);
-        need = t->scale_offset + 2ll * (t->dim / g);
+    if (t->quant == SCONE_QUANT_INT4) {
+        SCONE_REQUIRE(valid_int4_group(t->group), "%s: INT4 group %d must be a power of two >= 8", who, t->group);
+        SCONE_REQUIRE(t->dim % t->group == 0, "%s: dim %d not a multiple of group %d", who, t->dim, t->group);
     }
+    const int64_t payload = payload_bytes(t->quant, t->dim), scales = scale_bytes(t->quant, t->dim, t->group);
+    if (scales)  // the scales may sit anywhere past the payload, aligned
+        SCONE_REQUIRE(t->scale_offset >= payload && t->scale_offset % scale_align(t->quant) == 0, "%s: %s scale_offset %d invalid", who,
+                      t->quant == SCONE_QUANT_INT8 ? "INT8" : "INT4", t->scale_offset);
+    const int64_t need = scales ? t->scale_offset + scales : payload;
     SCONE_REQUIRE(t->row_stride >= need, "%s: row_stride %lld smaller than the %lld bytes a row needs", who,
                   (long long)t->row_stride, (long long)need);
     return SCONE_OK;
@@ -104,21 +98,6 @@ __global__ void __launch_bounds__(256) store_kernel(uint8_t *rows, int64_t row_s
     }
 }
 
-// 8 elements (chunk c) of a stored row in global memory -> fp32
-template <int QUANT>
-__device__ __forceinline__ void decode_row_chunk(const uint8_t *row, int c, int scale_off, int group_shift, f32x8 &x) {
-    if (QUANT == SCONE_QUANT_FP32) {
-        decode_fp32x8(ldg_stream_16(row + c * 32), ldg_stream_16(row + c * 32 + 16), x);
-    } else if (QUANT == SCONE_QUANT_FP16) {
-        decode_fp16x8(ldg_stream_16(row + c * 16), x);
-    } else if (QUANT == SCONE_QUANT_INT8) {
-        decode_int8x8(ldg_stream_8(row + c * 8), __ldg(reinterpret_cast<const float *>(row + scale_off)), x);
-    } else {
-        const __half hs = __ldg(reinterpret_cast<const __half *>(row + scale_off) + (c >> group_shift));
-        decode_int4x8(ldg_stream_4(row + c * 4), __half2float(hs), x);
-    }
-}
-
 // One warp per requested row: out[r] = dequant(table[ids[r]]) as fp32 / bf16 / fp16.
 template <int QUANT, int OUT>
 __global__ void __launch_bounds__(256) gather_kernel(const uint8_t *__restrict__ rows, int64_t row_stride, int64_t num_rows, int D,
@@ -132,20 +111,13 @@ __global__ void __launch_bounds__(256) gather_kernel(const uint8_t *__restrict__
     if (!ok && lane == 0 && status) atomicOr(status, SCONE_STATUS_TOKEN_OOR);
     const uint8_t *row = rows + (ok ? id : 0) * row_stride;
     const int nchunks = D >> 3;
-    constexpr int OB = OUT == SCONE_OUT_FP32 ? 4 : 2;
+    constexpr int OB = sizeof(OutChunk<OUT>) / 8;  // output bytes per element
+    const GlobalRows mem;
     for (int c = lane; c < nchunks; c += 32) {
         f32x8 x;
         if (!ok) zero8(x);
-        else decode_row_chunk<QUANT>(row, c, scale_off, group_shift, x);
-        uint8_t *o = out + ((int64_t)r * D + c * 8) * OB;
-        if (OUT == SCONE_OUT_FP32) {
-            *reinterpret_cast<float4 *>(o) = make_float4(x[0].x, x[0].y, x[1].x, x[1].y);
-            *reinterpret_cast<float4 *>(o + 16) = make_float4(x[2].x, x[2].y, x[3].x, x[3].y);
-        } else if (OUT == SCONE_OUT_BF16) {
-            *reinterpret_cast<uint4 *>(o) = pack_bf16x8(x);
-        } else {
-            *reinterpret_cast<uint4 *>(o) = pack_fp16x8(x);
-        }
+        else decode_chunk<QUANT>(load_chunk<QUANT>(mem, row, c, scale_off, group_shift, row_scale<QUANT>(mem, row, scale_off)), x);
+        *reinterpret_cast<OutChunk<OUT> *>(out + ((int64_t)r * D + c * 8) * OB) = pack_chunk<OUT>(x);
     }
 }
 
@@ -201,55 +173,23 @@ __global__ void __launch_bounds__(256) mean_kernel(const uint8_t *__restrict__ r
         }
     }
     const int nchunks = D >> 3;
-    constexpr int OB = OUT == SCONE_OUT_FP32 ? 4 : 2;
+    constexpr int OB = sizeof(OutChunk<OUT>) / 8;  // output bytes per element
+    const GlobalRows mem;
     for (int c = lane; c < nchunks; c += 32) {
         f32x8 acc;
         zero8(acc);
         for (int r = 0; r < k; ++r) {
+            const uint8_t *row = rows + (int64_t)ids[r] * row_stride;
             f32x8 x;
-            decode_row_chunk<QUANT>(rows + (int64_t)ids[r] * row_stride, c, scale_off, group_shift, x);
+            decode_chunk<QUANT>(load_chunk<QUANT>(mem, row, c, scale_off, group_shift, row_scale<QUANT>(mem, row, scale_off)), x);
             add8(acc, x);
         }
         if (k > 1) {
 #pragma unroll
             for (int e = 0; e < 4; ++e) acc[e] = make_float2(__fdiv_rn(acc[e].x, (float)k), __fdiv_rn(acc[e].y, (float)k));
         }
-        uint8_t *o = out + (t * D + c * 8) * OB;
-        if (OUT == SCONE_OUT_FP32) {
-            *reinterpret_cast<float4 *>(o) = make_float4(acc[0].x, acc[0].y, acc[1].x, acc[1].y);
-            *reinterpret_cast<float4 *>(o + 16) = make_float4(acc[2].x, acc[2].y, acc[3].x, acc[3].y);
-        } else if (OUT == SCONE_OUT_BF16) {
-            *reinterpret_cast<uint4 *>(o) = pack_bf16x8(acc);
-        } else {
-            *reinterpret_cast<uint4 *>(o) = pack_fp16x8(acc);
-        }
+        *reinterpret_cast<OutChunk<OUT> *>(out + (t * D + c * 8) * OB) = pack_chunk<OUT>(acc);
     }
-}
-
-template <int QUANT>
-static void launch_mean(int out_dtype, unsigned blocks, cudaStream_t stream, const scone_table_desc_t *t, int group_shift,
-                        const int32_t *all_ids, int max_n, int64_t T, int64_t L, void *out) {
-    const uint8_t *rows = static_cast<const uint8_t *>(t->d_rows);
-    uint8_t *o = static_cast<uint8_t *>(out);
-    if (out_dtype == SCONE_OUT_FP32)
-        mean_kernel<QUANT, SCONE_OUT_FP32><<<blocks, 256, 0, stream>>>(rows, t->row_stride, t->dim, group_shift, t->scale_offset, all_ids, max_n, T, L, o);
-    else if (out_dtype == SCONE_OUT_BF16)
-        mean_kernel<QUANT, SCONE_OUT_BF16><<<blocks, 256, 0, stream>>>(rows, t->row_stride, t->dim, group_shift, t->scale_offset, all_ids, max_n, T, L, o);
-    else
-        mean_kernel<QUANT, SCONE_OUT_FP16><<<blocks, 256, 0, stream>>>(rows, t->row_stride, t->dim, group_shift, t->scale_offset, all_ids, max_n, T, L, o);
-}
-
-template <int QUANT>
-static void launch_gather(int out_dtype, unsigned blocks, cudaStream_t stream, const scone_table_desc_t *t, int group_shift,
-                          const int64_t *ids, int64_t k, void *out, uint32_t *status) {
-    const uint8_t *rows = static_cast<const uint8_t *>(t->d_rows);
-    uint8_t *o = static_cast<uint8_t *>(out);
-    if (out_dtype == SCONE_OUT_FP32)
-        gather_kernel<QUANT, SCONE_OUT_FP32><<<blocks, 256, 0, stream>>>(rows, t->row_stride, t->num_rows, t->dim, group_shift, t->scale_offset, ids, k, o, status);
-    else if (out_dtype == SCONE_OUT_BF16)
-        gather_kernel<QUANT, SCONE_OUT_BF16><<<blocks, 256, 0, stream>>>(rows, t->row_stride, t->num_rows, t->dim, group_shift, t->scale_offset, ids, k, o, status);
-    else
-        gather_kernel<QUANT, SCONE_OUT_FP16><<<blocks, 256, 0, stream>>>(rows, t->row_stride, t->num_rows, t->dim, group_shift, t->scale_offset, ids, k, o, status);
 }
 
 }  // namespace scone
@@ -263,26 +203,13 @@ int scone_table_layout(int32_t quant, int32_t dim, int32_t group, int32_t align,
     SCONE_REQUIRE(dim > 0 && dim % 8 == 0, "scone_table_layout: dim %d must be a positive multiple of 8", dim);
     if (align <= 0) align = 32;
     SCONE_REQUIRE(align % 16 == 0, "scone_table_layout: align %d must be a multiple of 16", align);
-    int64_t bytes;
-    int32_t soff = 0;
-    if (quant == SCONE_QUANT_FP32) {
-        bytes = 4ll * dim;
-    } else if (quant == SCONE_QUANT_FP16) {
-        bytes = 2ll * dim;
-    } else if (quant == SCONE_QUANT_INT8) {
-        soff = dim;
-        bytes = dim + 4ll;
-    } else if (quant == SCONE_QUANT_INT4) {
-        SCONE_REQUIRE(group >= 8 && (group & (group - 1)) == 0 && dim % group == 0,
+    SCONE_REQUIRE(quant >= SCONE_QUANT_FP16 && quant <= SCONE_QUANT_FP32, "scone_table_layout: unknown quant %d", quant);
+    if (quant == SCONE_QUANT_INT4)
+        SCONE_REQUIRE(valid_int4_group(group) && dim % group == 0,
                       "scone_table_layout: INT4 needs a power-of-two group >= 8 dividing dim (group %d, dim %d)", group, dim);
-        soff = dim / 2;
-        bytes = dim / 2 + 2ll * (dim / group);
-    } else {
-        set_error("scone_table_layout: unknown quant %d", quant);
-        return SCONE_E_INVALID;
-    }
-    *row_stride = (bytes + align - 1) / align * align;
-    *scale_offset = soff;
+    const int64_t payload = payload_bytes(quant, dim), scales = scale_bytes(quant, dim, group);
+    *row_stride = (payload + scales + align - 1) / align * align;
+    *scale_offset = scales ? (int32_t)payload : 0;  // right after the payload, aligned as dim is a multiple of 8
     return SCONE_OK;
 }
 
@@ -300,14 +227,10 @@ int scone_table_store(const scone_table_desc_t *table, const float *d_rows_f32, 
                   (long long)row_base, (long long)(row_base + k));
     uint8_t *rows = static_cast<uint8_t *>(const_cast<void *>(table->d_rows));
     SCONE_GRID(blocks, (k + 7) / 8, "scone_table_store");
-    if (table->quant == SCONE_QUANT_FP32)
-        store_kernel<SCONE_QUANT_FP32><<<blocks, 256, 0, stream>>>(rows, table->row_stride, table->num_rows, table->dim, 0, 0, d_rows_f32, d_row_ids, row_base, k, nullptr);
-    else if (table->quant == SCONE_QUANT_FP16)
-        store_kernel<SCONE_QUANT_FP16><<<blocks, 256, 0, stream>>>(rows, table->row_stride, table->num_rows, table->dim, 0, 0, d_rows_f32, d_row_ids, row_base, k, nullptr);
-    else if (table->quant == SCONE_QUANT_INT8)
-        store_kernel<SCONE_QUANT_INT8><<<blocks, 256, 0, stream>>>(rows, table->row_stride, table->num_rows, table->dim, 0, table->scale_offset, d_rows_f32, d_row_ids, row_base, k, nullptr);
-    else
-        store_kernel<SCONE_QUANT_INT4><<<blocks, 256, 0, stream>>>(rows, table->row_stride, table->num_rows, table->dim, table->group, table->scale_offset, d_rows_f32, d_row_ids, row_base, k, nullptr);
+    with_constant<SCONE_QUANT_FP16, SCONE_QUANT_INT8, SCONE_QUANT_INT4, SCONE_QUANT_FP32>(table->quant, [&](auto q) {
+        store_kernel<q()><<<blocks, 256, 0, stream>>>(rows, table->row_stride, table->num_rows, table->dim, table->group, table->scale_offset,
+                                                      d_rows_f32, d_row_ids, row_base, k, nullptr);
+    });
     SCONE_LAUNCHED();
     return SCONE_OK;
 }
@@ -327,14 +250,14 @@ int scone_embed_mean_forward(const scone_index_t *index, const scone_table_desc_
     SCONE_REQUIRE(ix->n <= table->num_rows, "scone_embed_mean_forward: index has more f-grams than the table has rows");
     rc = scone_index_match_all(index, d_ids, B, L, d_work, stream_);
     if (rc != SCONE_OK) return rc;
-    int group_shift = 0;
-    if (table->quant == SCONE_QUANT_INT4)
-        while ((1 << group_shift) < table->group / 8) ++group_shift;
     SCONE_GRID(blocks, (T + 7) / 8, "scone_embed_mean_forward");
-    if (table->quant == SCONE_QUANT_FP32) launch_mean<SCONE_QUANT_FP32>(out_dtype, blocks, stream, table, group_shift, d_work, ix->max_n, T, L, d_out);
-    else if (table->quant == SCONE_QUANT_FP16) launch_mean<SCONE_QUANT_FP16>(out_dtype, blocks, stream, table, group_shift, d_work, ix->max_n, T, L, d_out);
-    else if (table->quant == SCONE_QUANT_INT8) launch_mean<SCONE_QUANT_INT8>(out_dtype, blocks, stream, table, group_shift, d_work, ix->max_n, T, L, d_out);
-    else launch_mean<SCONE_QUANT_INT4>(out_dtype, blocks, stream, table, group_shift, d_work, ix->max_n, T, L, d_out);
+    with_constant<SCONE_QUANT_FP16, SCONE_QUANT_INT8, SCONE_QUANT_INT4, SCONE_QUANT_FP32>(table->quant, [&](auto q) {
+        with_constant<SCONE_OUT_BF16, SCONE_OUT_FP16, SCONE_OUT_FP32>(out_dtype, [&](auto o) {
+            mean_kernel<q(), o()><<<blocks, 256, 0, stream>>>(static_cast<const uint8_t *>(table->d_rows), table->row_stride, table->dim,
+                                                              group_shift(table->group), table->scale_offset, d_work, ix->max_n, T, L,
+                                                              static_cast<uint8_t *>(d_out));
+        });
+    });
     SCONE_LAUNCHED();
     return SCONE_OK;
 }
@@ -366,14 +289,14 @@ int scone_table_gather(const scone_table_desc_t *table, const int64_t *d_row_ids
     SCONE_REQUIRE(k >= 0, "scone_table_gather: negative k");
     if (k == 0) return SCONE_OK;
     SCONE_REQUIRE(d_row_ids && d_out, "scone_table_gather: NULL buffer");
-    int group_shift = 0;
-    if (table->quant == SCONE_QUANT_INT4)
-        while ((1 << group_shift) < table->group / 8) ++group_shift;
     SCONE_GRID(blocks, (k + 7) / 8, "scone_table_gather");
-    if (table->quant == SCONE_QUANT_FP32) launch_gather<SCONE_QUANT_FP32>(out_dtype, blocks, stream, table, group_shift, d_row_ids, k, d_out, d_status);
-    else if (table->quant == SCONE_QUANT_FP16) launch_gather<SCONE_QUANT_FP16>(out_dtype, blocks, stream, table, group_shift, d_row_ids, k, d_out, d_status);
-    else if (table->quant == SCONE_QUANT_INT8) launch_gather<SCONE_QUANT_INT8>(out_dtype, blocks, stream, table, group_shift, d_row_ids, k, d_out, d_status);
-    else launch_gather<SCONE_QUANT_INT4>(out_dtype, blocks, stream, table, group_shift, d_row_ids, k, d_out, d_status);
+    with_constant<SCONE_QUANT_FP16, SCONE_QUANT_INT8, SCONE_QUANT_INT4, SCONE_QUANT_FP32>(table->quant, [&](auto q) {
+        with_constant<SCONE_OUT_BF16, SCONE_OUT_FP16, SCONE_OUT_FP32>(out_dtype, [&](auto o) {
+            gather_kernel<q(), o()><<<blocks, 256, 0, stream>>>(static_cast<const uint8_t *>(table->d_rows), table->row_stride, table->num_rows,
+                                                                table->dim, group_shift(table->group), table->scale_offset, d_row_ids, k,
+                                                                static_cast<uint8_t *>(d_out), d_status);
+        });
+    });
     SCONE_LAUNCHED();
     return SCONE_OK;
 }

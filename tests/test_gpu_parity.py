@@ -708,6 +708,24 @@ def test_reference_code_mean_mode_golden():
             np.testing.assert_allclose(g[b], w, rtol=0, atol=1e-8)
 
 
+@pytest.mark.parametrize("quant", ["fp32", "fp16", "int8", "int4"])
+def test_mean_mode_16bit_outputs_are_the_rounded_fp32_output(quant):
+    """The mean kernel computes each fp32 mean once and rounds it to the output type: its bf16 / fp16 outputs are bit for bit
+    the round-to-nearest-even cast of its fp32 output on the same inputs, for every stored format."""
+    sb, S = _mods()
+    toks, lens = S.make_vocab_numpy(1500, 5, 120, seed=71, min_n=1)
+    rows = S.make_rows_numpy(1500, 264, seed=72)                 # 33 chunks: one lane takes two
+    qq = torch.from_numpy(S.make_stream_numpy(toks, lens, 3, 90, 120, seed=73)).to(DEV)
+    ix = _index(toks, lens)
+    t = sb.CacheTable(1500, 264, quant, group=8 if quant == "int4" else 128)
+    t.store(torch.from_numpy(rows).to(DEV))
+    g32 = sb.embed_mean_forward(ix, t, qq).cpu().numpy()
+    assert np.count_nonzero(g32) > g32.size // 2
+    for name, dt in TORCH_DT.items():
+        g16 = _bits(sb.embed_mean_forward(ix, t, qq, dtype=dt))
+        assert np.array_equal(g16, po.cast_bits(g32, name)), name
+
+
 def test_host_pipeline_matches_direct_call():
     sb, S = _mods()
     toks, lens = S.make_vocab_numpy(3000, 4, 300, seed=71)

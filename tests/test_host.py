@@ -257,6 +257,47 @@ def test_c_abi_rejects_bad_arguments_without_a_gpu():
     assert b"k too large" in L.scone_last_error()
 
 
+def test_every_table_layout_is_accepted_by_the_table_check():
+    """scone_table_layout and the descriptor check of every table entry point state one row-format rule: each layout is
+    accepted, a row_stride 16 bytes short of the row is refused, and INT8 / INT4 scales may sit at any aligned offset past
+    the payload.  check_table runs before scone_table_gather's k == 0 return, so no call reaches the device."""
+    import ctypes as C
+    from scone_b200 import _lib
+    L = _lib.load()
+    rows = 16                                                    # aligned stand-in pointer, never read
+
+    def layout(quant, dim, group, align):
+        rs, so = C.c_int64(), C.c_int32()
+        assert L.scone_table_layout(quant, dim, group, align, C.byref(rs), C.byref(so)) == 0, L.scone_last_error()
+        return rs.value, so.value
+
+    def check(quant, dim, group, stride, soff):
+        desc = _lib.TableDesc(rows, stride, 1000, quant, dim, group, soff)
+        return L.scone_table_gather(C.byref(desc), None, 0, None, _lib.OUT_FP32, None, None)
+
+    cases = 0
+    for name, quant in _lib.QUANT.items():
+        for dim in (8, 64, 136, 1024, 4096, 16384):
+            groups = [g for g in (8, 16, 32, 64, 128, 256) if dim % g == 0] if name == "int4" else [128]
+            for group in groups:
+                tight, soff = layout(quant, dim, group, 16)      # the smallest 16-byte multiple that holds the row
+                for align in (16, 32, 128):
+                    stride, soff_a = layout(quant, dim, group, align)
+                    assert soff_a == soff and stride % align == 0 and tight <= stride < tight + align
+                    assert check(quant, dim, group, stride, soff) == 0, (name, dim, group, align, L.scone_last_error())
+                    cases += 1
+                assert check(quant, dim, group, tight - 16, soff) == _lib.E_INVALID, (name, dim, group)
+                assert b"row_stride" in L.scone_last_error()
+                if name in ("int8", "int4"):
+                    salign = 4 if name == "int8" else 2
+                    roomy = tight + 128                          # room for the scales wherever they move
+                    assert check(quant, dim, group, roomy, soff + salign) == 0, (name, dim, group)
+                    for bad in (soff - salign, soff + 1):       # below the payload / misaligned
+                        assert check(quant, dim, group, roomy, bad) == _lib.E_INVALID, (name, dim, group, bad)
+                        assert b"scale_offset" in L.scone_last_error()
+    assert cases == 3 * (3 * 6 + 24)
+
+
 def test_bench_reference_arm_runs_on_cpu():
     """`bench.py --impl reference` (the CPU arm) needs no GPU and prints the contract's JSON line."""
     import json

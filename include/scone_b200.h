@@ -67,8 +67,8 @@ typedef struct scone_index_info {
     int32_t max_n;
     uint32_t len_mask;   /* bit (n-1) set when some f-gram has length n */
     int32_t max_probe;   /* longest insert probe sequence seen at build time */
-    int32_t slot_bytes;  /* 32, or 16 for the compact formats (all tokens < 65535 and max_n <= 6; or all tokens < 1048575,
-                            max_n <= 5 and fewer than 2^28 - 1 f-grams) */
+    int32_t slot_bytes;  /* 32 for the wide format, 16 for compact-16 (every token < 65535, max_n <= 6) and compact-20
+                            (every token < 1048575, max_n <= 5, fewer than 2^28 - 1 f-grams) */
     int64_t filter_bytes; /* bytes of the L2-resident pre-filter (included in `bytes`), 0 = none */
     int32_t slot_format;  /* 0 = 32-byte slots, 1 = compact 16-byte (six 16-bit tokens), 2 = compact 16-byte (five 20-bit tokens) */
     int32_t reserved;
@@ -97,13 +97,18 @@ const char *scone_last_error(void);
  * d_tokens: int32 [n, max_n], f-gram r in row r in reading order, padded with -1.
  * d_lens  : uint8 [n].  The id of an f-gram is its row number (frequency rank in the
  *           reference, n_gram_extractor.py:98-99).
- * The open-addressing table (32-byte slots, key stored inline, home slot from a
- * rolling 64-bit hash) is built by kernels on `stream`; the call then reads back a
- * build audit and fails with SCONE_E_VOCAB if two rows hold the same f-gram, a length
- * is outside [1, max_n] or a token is negative.  When every token is < 65535 and max_n <= 6 the compact
- * 16-byte slot format is used (four slots per 64-byte probe).  load_factor in (0, 0.9]; <= 0 -> 0.25 (128 B of
- * index per f-gram with 32-byte slots, 64 B with compact slots): short probe chains matter more than index size,
- * see DESIGN.md. */
+ * The open-addressing table (key stored inline, home slot from a rolling 64-bit hash)
+ * is built by kernels on `stream`; the call then reads back a build audit and fails
+ * with SCONE_E_VOCAB if two rows hold the same f-gram, a length is outside [1, max_n]
+ * or a token is negative.  The slot format is compact-16 if it holds the vocabulary, else
+ * compact-20 if it does, else wide:
+ *   compact-16: 16 bytes, id + six 16-bit tokens: every token < 65535 and max_n <= 6;
+ *   compact-20: 16 bytes, 28-bit id + five 20-bit tokens: every token < 1048575, max_n <= 5
+ *               and fewer than 2^28 - 1 f-grams;
+ *   wide:       32 bytes, id + seven int32 tokens: any vocabulary.
+ * A probe step reads one 64-byte block: four compact slots or two wide ones.  load_factor in
+ * (0, 0.9]; <= 0 -> 0.25 (128 B of index per f-gram with 32-byte slots, 64 B with 16-byte
+ * slots): short probe chains matter more than index size, see DESIGN.md. */
 int scone_index_create(const int32_t *d_tokens, const uint8_t *d_lens, int64_t n, int32_t max_n,
                        double load_factor, void *stream, scone_index_t **out);
 int scone_index_destroy(scone_index_t *index);

@@ -105,7 +105,7 @@ static int embed_forward_impl(const scone_index_t *index, const scone_table_desc
     if (rc != SCONE_OK) return rc;
     p.additive = (flags & SCONE_EMBED_ADDITIVE) ? 1 : 0;
     p.flags = flags;
-    return dispatch(lanes_per_position(ix->len_mask, ix->max_n), false, p, table->quant, out_dtype, (cudaStream_t)stream_);
+    return dispatch(lanes_per_position(ix->v.len_mask, ix->v.max_n), false, p, table->quant, out_dtype, (cudaStream_t)stream_);
 }
 
 int scone_embed_forward(const scone_index_t *index, const scone_table_desc_t *table, const void *d_base_emb, int64_t base_rows,
@@ -154,7 +154,7 @@ int scone_embed_forward_sharded(const scone_index_t *index, const scone_table_de
     p.rows = nullptr;
     p.num_rows = total_rows;
     p.world = -world;  // negative: always go through the pointer table, even for one shard
-    return dispatch(lanes_per_position(ix->len_mask, ix->max_n), false, p, shard->quant, out_dtype, (cudaStream_t)stream_);
+    return dispatch(lanes_per_position(ix->v.len_mask, ix->v.max_n), false, p, shard->quant, out_dtype, (cudaStream_t)stream_);
 }
 
 int scone_embed_gather(const scone_table_desc_t *table, const void *d_base_emb, int64_t base_rows, const void *d_pos_emb,

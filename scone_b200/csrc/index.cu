@@ -4,9 +4,7 @@
 // (scone/tokenization/n_gram_extractor.py:41-44, :96-99, :121-122) and the tuple -> id lookup of
 // scone/inference/embedding_cache.py:173.
 #include <cstdlib>
-#include <cstring>
 
-#include "common.cuh"
 #include "match.cuh"
 
 namespace scone {
@@ -21,38 +19,12 @@ struct BuildStats {
     int max_tok;
 };
 
-// First pass: validate the vocabulary and find the largest token (decides the slot format).
-__global__ void __launch_bounds__(256) index_scan_kernel(const int32_t *__restrict__ tokens, const uint8_t *__restrict__ lens, int64_t n,
-                                                         int32_t max_n, BuildStats *stats) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+// Key and hash of vocabulary row i; returns its length, 0 for a length outside [1, max_n], -1 for a negative token.
+__device__ __forceinline__ int vocab_key(const int32_t *__restrict__ tokens, const uint8_t *__restrict__ lens, int64_t i, int32_t max_n,
+                                         int32_t (&key)[7], uint64_t &h) {
     const int len = lens[i];
-    if (len < 1 || len > max_n) {
-        atomicAdd(&stats->bad_len, 1ull);
-        return;
-    }
-    int mx = 0;
-    bool bad = false;
-    for (int k = 0; k < len; ++k) {
-        const int32_t t = tokens[i * max_n + k];
-        bad |= t < 0;
-        mx = t > mx ? t : mx;
-    }
-    if (bad) atomicAdd(&stats->bad_tok, 1ull);
-    else atomicMax(&stats->max_tok, mx);
-}
-
-// One thread per f-gram: claim the first free slot of its probe sequence with a CAS on the id
-// word, then fill in the key.  No lookup runs concurrently with the build.
-__global__ void __launch_bounds__(256) index_build_kernel(const int32_t *__restrict__ tokens, const uint8_t *__restrict__ lens,
-                                                          int64_t n, int32_t max_n, Slot *slots, uint64_t cap, int compact,
-                                                          uint32_t *filter, uint32_t filter_mask, BuildStats *stats) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const int len = lens[i];
-    if (len < 1 || len > max_n) return;  // counted by the scan
-    int32_t key[7];
-    uint64_t h = hash_seed();
+    if (len < 1 || len > max_n) return 0;
+    h = hash_seed();
     bool bad = false;
 #pragma unroll
     for (int k = 0; k < 7; ++k) {
@@ -64,47 +36,42 @@ __global__ void __launch_bounds__(256) index_build_kernel(const int32_t *__restr
             h = hash_roll(h, (uint32_t)t);
         }
     }
-    if (bad) return;  // counted by the scan
+    if (bad) return -1;
     h = hash_finish(h, len);
-    if (filter) atomicOr(&filter[filter_word(h, filter_mask)], filter_bits(h));
-    int probes = 1;
-    if (compact == kSlotCompact20) {
-        Slot20 *s20 = reinterpret_cast<Slot20 *>(slots);
-        uint32_t k20[4];
-        pack_key20(key, k20);  // validity was established by the scan pass (max token, max_n)
-        uint64_t s = home_slot16(h, cap);
-        for (;;) {
-            uint32_t old = atomicCAS(&s20[s].w[0], kEmpty20, (uint32_t)i | k20[0]);
-            if (old == kEmpty20) break;
-            if (++s == cap) s = 0;
-            ++probes;
-        }
-#pragma unroll
-        for (int k = 1; k < 4; ++k) s20[s].w[k] = k20[k];
-    } else if (compact == kSlotCompact16) {
-        Slot16 *s16 = reinterpret_cast<Slot16 *>(slots);
-        uint64_t s = home_slot16(h, cap);
-        for (;;) {
-            int32_t old = atomicCAS(&s16[s].id, -1, (int32_t)i);
-            if (old == -1) break;
-            if (++s == cap) s = 0;
-            ++probes;
-        }
-        uint32_t k16[3];
-        pack_key16(key, k16);
-#pragma unroll
-        for (int k = 0; k < 3; ++k) s16[s].t[k] = k16[k];
-    } else {
-        uint64_t s = home_slot(h, cap);
-        for (;;) {
-            int32_t old = atomicCAS(&slots[s].w[0], -1, (int32_t)i);
-            if (old == -1) break;
-            if (++s == cap) s = 0;
-            ++probes;
-        }
-#pragma unroll
-        for (int k = 0; k < 7; ++k) slots[s].w[k + 1] = key[k];
+    return len;
+}
+
+// First pass: validate the vocabulary and find the largest token (decides the slot format).
+__global__ void __launch_bounds__(256) index_scan_kernel(const int32_t *__restrict__ tokens, const uint8_t *__restrict__ lens, int64_t n,
+                                                         int32_t max_n, BuildStats *stats) {
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int32_t key[7];
+    uint64_t h;
+    const int len = vocab_key(tokens, lens, i, max_n, key, h);
+    if (len <= 0) {
+        atomicAdd(len == 0 ? &stats->bad_len : &stats->bad_tok, 1ull);
+        return;
     }
+    int mx = 0;
+#pragma unroll
+    for (int k = 0; k < 7; ++k) mx = key[k] > mx ? key[k] : mx;
+    atomicMax(&stats->max_tok, mx);
+}
+
+// One thread per f-gram: set its filter bits and insert it.
+__global__ void __launch_bounds__(256) index_build_kernel(const int32_t *__restrict__ tokens, const uint8_t *__restrict__ lens,
+                                                          int64_t n, int32_t max_n, IndexView ix, BuildStats *stats) {
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int32_t key[7];
+    uint64_t h;
+    const int len = vocab_key(tokens, lens, i, max_n, key, h);
+    if (len <= 0) return;  // counted by the scan
+    if (ix.filter) atomicOr(&ix.filter[filter_word(h, ix.filter_mask)], filter_bits(h));
+    const int probes = ix.format == kSlotCompact20   ? insert<Compact20Slot>(ix.slots, ix.cap, h, key, (uint32_t)i)
+                       : ix.format == kSlotCompact16 ? insert<Compact16Slot>(ix.slots, ix.cap, h, key, (uint32_t)i)
+                                                     : insert<WideSlot>(ix.slots, ix.cap, h, key, (uint32_t)i);
     atomicOr(&stats->len_mask, 1u << (len - 1));
     atomicMax(&stats->max_probe, probes);
 }
@@ -115,21 +82,9 @@ __global__ void __launch_bounds__(256) index_audit_kernel(const int32_t *__restr
                                                           int64_t n, int32_t max_n, IndexView ix, BuildStats *stats) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const int len = lens[i];
-    if (len < 1 || len > max_n) return;
     int32_t key[7];
-    uint64_t h = hash_seed();
-#pragma unroll
-    for (int k = 0; k < 7; ++k) {
-        key[k] = -1;
-        if (k < len) {
-            int32_t t = tokens[i * max_n + (len - 1 - k)];
-            if (t < 0) return;
-            key[k] = t;
-            h = hash_roll(h, (uint32_t)t);
-        }
-    }
-    h = hash_finish(h, len);
+    uint64_t h;
+    if (vocab_key(tokens, lens, i, max_n, key, h) <= 0) return;
     if (probe_any(ix, h, key) != (int32_t)i) atomicAdd(&stats->dup, 1ull);
 }
 
@@ -181,7 +136,7 @@ int scone_index_create(const int32_t *d_tokens, const uint8_t *d_lens, int64_t n
     cudaStream_t stream = (cudaStream_t)stream_;
     SCONE_REQUIRE(out != nullptr, "scone_index_create: out is NULL");
     *out = nullptr;
-    SCONE_REQUIRE(n >= 0 && n < (int64_t)0x7FFFFFFF, "scone_index_create: n = %lld outside [0, 2^31-1)", (long long)n);
+    SCONE_REQUIRE(n >= 0 && n < kSlotFormats[kSlotWide].n_limit, "scone_index_create: n = %lld outside [0, 2^31-1)", (long long)n);
     SCONE_REQUIRE(max_n >= 1 && max_n <= SCONE_MAX_N, "scone_index_create: max_n = %d outside [1, %d]", max_n, SCONE_MAX_N);
     SCONE_REQUIRE(n == 0 || (d_tokens && d_lens), "scone_index_create: NULL vocabulary arrays");
     SCONE_REQUIRE(!(load_factor > 0.9), "scone_index_create: load_factor %.3f > 0.9", load_factor);
@@ -192,12 +147,11 @@ int scone_index_create(const int32_t *d_tokens, const uint8_t *d_lens, int64_t n
         return SCONE_E_NOMEM;
     }
     ix->n = n;
-    ix->max_n = max_n;
+    ix->v.max_n = max_n;
     BuildStats *d_stats = nullptr;
     BuildStats h{};
     const unsigned blocks = (unsigned)((n + 255) / 256);
     int rc = [&]() -> int {
-        SCONE_CUDA(cudaGetDevice(&ix->device));
         SCONE_CUDA(cudaMalloc(&d_stats, sizeof(BuildStats)));
         SCONE_CUDA(cudaMemsetAsync(d_stats, 0, sizeof(BuildStats), stream));
         // pass 1: validate, find the largest token -> slot format
@@ -208,66 +162,32 @@ int scone_index_create(const int32_t *d_tokens, const uint8_t *d_lens, int64_t n
         SCONE_CUDA(cudaMemcpyAsync(&h, d_stats, sizeof h, cudaMemcpyDeviceToHost, stream));
         SCONE_CUDA(cudaStreamSynchronize(stream));
         if (h.bad_len || h.bad_tok) return SCONE_OK;  // reported below
-        const char *fmt = getenv("SCONE_INDEX_FORMAT");  // "wide" / "compact" / "compact20" override the automatic choice (testing)
-        const bool fits16 = max_n <= 6 && h.max_tok < 0xFFFF;
-        const bool fits20 = max_n <= 5 && h.max_tok < (int)kPad20 && n < (int64_t)kIdMask20;
-        ix->compact = fits16 ? kSlotCompact16 : fits20 ? kSlotCompact20 : kSlotWide;
-        if (fmt && !strcmp(fmt, "wide")) ix->compact = kSlotWide;
-        if (fmt && !strcmp(fmt, "compact")) {
-            if (!fits16) {
-                set_error("scone_index_create: SCONE_INDEX_FORMAT=compact needs max_n <= 6 and tokens < 65535");
-                return SCONE_E_INVALID;
-            }
-            ix->compact = kSlotCompact16;
-        }
-        if (fmt && !strcmp(fmt, "prefer-compact20") && fits20) ix->compact = kSlotCompact20;  // testing: small vocabularies too
-        if (fmt && !strcmp(fmt, "compact20")) {
-            if (!fits20) {
-                set_error("scone_index_create: SCONE_INDEX_FORMAT=compact20 needs max_n <= 5, tokens < 1048575 and n < 2^28 - 1");
-                return SCONE_E_INVALID;
-            }
-            ix->compact = kSlotCompact20;
-        }
-        // default load factor 0.25 for both formats (measured: compact at 0.5 costs config 1 a microsecond of probe chain)
-        const double lf = load_factor > 0.0 ? load_factor : 0.25;
-        uint64_t cap = (uint64_t)((double)n / lf) + 1;
-        if (cap < 64) cap = 64;
-        cap = (cap + 3) & ~3ull;  // whole 64-byte blocks of either format
-        ix->cap = cap;
-        const size_t bytes = cap * (ix->compact ? sizeof(Slot16) : sizeof(Slot));
-        cudaError_t e = cudaMalloc(&ix->slots, bytes);
-        if (e != cudaSuccess) {
-            set_error("scone_index_create: cudaMalloc of %llu slot bytes failed: %s", (unsigned long long)bytes, cudaGetErrorString(e));
-            ix->slots = nullptr;
-            return e == cudaErrorMemoryAllocation ? SCONE_E_NOMEM : SCONE_E_CUDA;
-        }
-        SCONE_CUDA(cudaMemsetAsync(ix->slots, 0xFF, bytes, stream));
-        // pre-filter (common.cuh: filter_pass): 16 bits per f-gram up to 12 M f-grams (24 MB), 8 bits up to 48 M (48 MB), none
-        // above -- it only pays while it stays in L2; SCONE_INDEX_FILTER=never / always override (testing)
-        const char *fenv = getenv("SCONE_INDEX_FILTER");
-        const bool f_never = fenv && !strcmp(fenv, "never"), f_always = fenv && !strcmp(fenv, "always");
-        if (n > 0 && !f_never && (f_always || n <= 48000000ll)) {
-            uint64_t words = (uint64_t)(n <= 12000000ll ? (n + 1) / 2 : (n + 3) / 4);
-            if (words < 1024) words = 1024;
-            words = (words + 31) & ~31ull;
-            e = cudaMalloc(&ix->filter, words * sizeof(uint32_t));
+        const IndexPlan pl = plan_index(
+            IndexCall{n, max_n, h.max_tok, load_factor, getenv("SCONE_INDEX_FORMAT"), getenv("SCONE_INDEX_FILTER")});
+        ix->v.format = pl.format;
+        ix->v.cap = pl.cap;
+        ix->v.filter_mask = pl.filter_words;
+        ix->filter_always = pl.filter_always;
+        // device buffer filled with `fill` bytes; the pointer stays NULL when the allocation fails
+        auto alloc = [&](auto **p, size_t bytes, int fill, const char *what) -> int {
+            cudaError_t e = cudaMalloc(p, bytes);
             if (e != cudaSuccess) {
-                set_error("scone_index_create: cudaMalloc of %llu filter bytes failed: %s", (unsigned long long)(words * 4), cudaGetErrorString(e));
-                ix->filter = nullptr;
+                set_error("scone_index_create: cudaMalloc of %llu %s bytes failed: %s", (unsigned long long)bytes, what, cudaGetErrorString(e));
+                *p = nullptr;
                 return e == cudaErrorMemoryAllocation ? SCONE_E_NOMEM : SCONE_E_CUDA;
             }
-            ix->filter_mask = (uint32_t)words;
-            ix->filter_always = f_always ? 1 : 0;
-            SCONE_CUDA(cudaMemsetAsync(ix->filter, 0, words * sizeof(uint32_t), stream));
-        }
-        // pass 2: insert, then every f-gram looks itself up (duplicate audit)
+            SCONE_CUDA(cudaMemsetAsync(*p, fill, bytes, stream));
+            return SCONE_OK;
+        };
+        int rc = alloc(&ix->v.slots, pl.cap * kSlotFormats[pl.format].slot_bytes, 0xFF, "slot");  // all-ones: every slot empty
+        if (rc == SCONE_OK && pl.filter_words) rc = alloc(&ix->v.filter, (size_t)pl.filter_words * sizeof(uint32_t), 0, "filter");
+        if (rc != SCONE_OK) return rc;
+        // pass 2: insert, then every f-gram looks itself up (duplicate audit).  Both read the handle's view (its len_mask is
+        // not set yet), with the filter: an f-gram the filter rejected would not find itself.
         if (n > 0) {
-            index_build_kernel<<<blocks, 256, 0, stream>>>(d_tokens, d_lens, n, max_n, ix->slots, cap, ix->compact, ix->filter,
-                                                           ix->filter_mask, d_stats);
+            index_build_kernel<<<blocks, 256, 0, stream>>>(d_tokens, d_lens, n, max_n, ix->v, d_stats);
             SCONE_LAUNCHED();
-            // the audit goes through the filter too: an f-gram the filter rejected would not find itself
-            IndexView v{ix->slots, cap, 0xFFFFFFFFu, max_n, ix->compact, ix->filter, ix->filter_mask};
-            index_audit_kernel<<<blocks, 256, 0, stream>>>(d_tokens, d_lens, n, max_n, v, d_stats);
+            index_audit_kernel<<<blocks, 256, 0, stream>>>(d_tokens, d_lens, n, max_n, ix->v, d_stats);
             SCONE_LAUNCHED();
         }
         SCONE_CUDA(cudaMemcpyAsync(&h, d_stats, sizeof h, cudaMemcpyDeviceToHost, stream));
@@ -281,12 +201,12 @@ int scone_index_create(const int32_t *d_tokens, const uint8_t *d_lens, int64_t n
         rc = SCONE_E_VOCAB;
     }
     if (rc != SCONE_OK) {
-        if (ix->slots) cudaFree(ix->slots);
-        if (ix->filter) cudaFree(ix->filter);
+        if (ix->v.slots) cudaFree(ix->v.slots);
+        if (ix->v.filter) cudaFree(ix->v.filter);
         delete ix;
         return rc;
     }
-    ix->len_mask = h.len_mask;
+    ix->v.len_mask = h.len_mask;
     ix->max_probe = h.max_probe;
     *out = reinterpret_cast<scone_index_t *>(ix);
     return SCONE_OK;
@@ -295,11 +215,9 @@ int scone_index_create(const int32_t *d_tokens, const uint8_t *d_lens, int64_t n
 int scone_index_destroy(scone_index_t *index) {
     if (!index) return SCONE_OK;
     scone_index_impl *ix = reinterpret_cast<scone_index_impl *>(index);
-    cudaError_t e = cudaFree(ix->slots);
-    if (ix->filter) {
-        cudaError_t e2 = cudaFree(ix->filter);
-        if (e == cudaSuccess) e = e2;
-    }
+    cudaError_t e = cudaFree(ix->v.slots);
+    const cudaError_t e2 = cudaFree(ix->v.filter);  // NULL (no filter) frees nothing
+    if (e == cudaSuccess) e = e2;
     delete ix;
     if (e != cudaSuccess) {
         set_error("scone_index_destroy: cudaFree failed: %s", cudaGetErrorString(e));
@@ -312,14 +230,14 @@ int scone_index_info(const scone_index_t *index, scone_index_info_t *info) {
     SCONE_REQUIRE(index && info, "scone_index_info: NULL argument");
     const scone_index_impl *ix = reinterpret_cast<const scone_index_impl *>(index);
     info->num_fgrams = ix->n;
-    info->capacity = (int64_t)ix->cap;
-    info->filter_bytes = ix->filter ? (int64_t)ix->filter_mask * 4 : 0;
-    info->bytes = (int64_t)(ix->cap * (ix->compact ? sizeof(Slot16) : sizeof(Slot))) + info->filter_bytes;
-    info->max_n = ix->max_n;
-    info->len_mask = ix->len_mask;
+    info->capacity = (int64_t)ix->v.cap;
+    info->filter_bytes = ix->v.filter ? (int64_t)ix->v.filter_mask * 4 : 0;
+    info->slot_bytes = kSlotFormats[ix->v.format].slot_bytes;
+    info->bytes = (int64_t)ix->v.cap * info->slot_bytes + info->filter_bytes;
+    info->max_n = ix->v.max_n;
+    info->len_mask = ix->v.len_mask;
     info->max_probe = ix->max_probe;
-    info->slot_bytes = (int32_t)(ix->compact ? sizeof(Slot16) : sizeof(Slot));
-    info->slot_format = ix->compact;
+    info->slot_format = ix->v.format;
     return SCONE_OK;
 }
 
@@ -334,7 +252,7 @@ int scone_index_lookup(const scone_index_t *index, const int64_t *d_ids, int64_t
     SCONE_REQUIRE(T < (1ll << 40), "scone_index_lookup: batch too large");
     const scone_index_impl *ix = reinterpret_cast<const scone_index_impl *>(index);
     IndexView v = view_of(ix, T);
-    const int P = lanes_per_position(ix->len_mask, ix->max_n);
+    const int P = lanes_per_position(ix->v.len_mask, ix->v.max_n);
     const int64_t windows = (T + (32 / P) - 1) / (32 / P);
     SCONE_GRID(blocks, (windows + 7) / 8, "scone_index_lookup");
     switch (P) {
@@ -357,7 +275,7 @@ int scone_index_match_all(const scone_index_t *index, const int64_t *d_ids, int6
     SCONE_REQUIRE(d_ids && d_out, "scone_index_match_all: NULL buffer");
     const scone_index_impl *ix = reinterpret_cast<const scone_index_impl *>(index);
     IndexView v = view_of(ix, T);
-    const int P = lanes_dense(ix->max_n);
+    const int P = lanes_dense(ix->v.max_n);
     const int64_t windows = (T + (32 / P) - 1) / (32 / P);
     SCONE_GRID(blocks, (windows + 7) / 8, "scone_index_match_all");
     switch (P) {

@@ -5,7 +5,7 @@
 // at position base + j; the P candidates of a position are resolved concurrently and the longest
 // hit is picked with one ballot (Algorithm 2: n = max_n .. 1, first hit wins).
 #pragma once
-#include "common.cuh"
+#include "index_format.cuh"
 
 namespace scone {
 

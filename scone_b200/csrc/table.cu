@@ -4,6 +4,7 @@
 // get_embeddings gather (:113-147).  The reference keeps fp32 rows; the three stored formats and
 // their formulas are defined in oracle/py_oracle.py (SURVEY.md section 8c) and implemented here
 // with the same fp32 operations in the same order, so the stored bits are identical.
+#include "index_format.cuh"
 #include "row_format.cuh"
 
 namespace scone {
@@ -254,7 +255,7 @@ int scone_embed_mean_forward(const scone_index_t *index, const scone_table_desc_
     with_constant<SCONE_QUANT_FP16, SCONE_QUANT_INT8, SCONE_QUANT_INT4, SCONE_QUANT_FP32>(table->quant, [&](auto q) {
         with_constant<SCONE_OUT_BF16, SCONE_OUT_FP16, SCONE_OUT_FP32>(out_dtype, [&](auto o) {
             mean_kernel<q(), o()><<<blocks, 256, 0, stream>>>(static_cast<const uint8_t *>(table->d_rows), table->row_stride, table->dim,
-                                                              group_shift(table->group), table->scale_offset, d_work, ix->max_n, T, L,
+                                                              group_shift(table->group), table->scale_offset, d_work, ix->v.max_n, T, L,
                                                               static_cast<uint8_t *>(d_out));
         });
     });

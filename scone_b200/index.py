@@ -19,6 +19,10 @@ def _require_cuda(t: torch.Tensor, name: str) -> None:
         raise ValueError(f"{name} must be a CUDA tensor: scone_b200 has no CPU path")
 
 
+# scone_index_info_t::slot_format -> name, in the order of index_plan.h's SlotFormat (kSlotFormats[].name)
+SLOT_FORMATS = ("wide32", "compact16", "compact20")
+
+
 class FGramIndex:
     """Open-addressing hash index of the f-gram vocabulary in HBM.
 
@@ -54,7 +58,7 @@ class FGramIndex:
         self.capacity, self.bytes = int(info.capacity), int(info.bytes)
         self.len_mask, self.max_probe = int(info.len_mask), int(info.max_probe)
         self.slot_bytes = int(info.slot_bytes)
-        self.slot_format = ("wide32", "compact16", "compact20")[int(info.slot_format)]
+        self.slot_format = SLOT_FORMATS[int(info.slot_format)]
         self.filter_bytes = int(info.filter_bytes)     # L2-resident pre-filter (0 = none), included in `bytes`
 
     @property

@@ -1,8 +1,8 @@
 """Host-side driver of the launch plans of the fused path (scone_b200/csrc/embed_plan.h) and of the projection fold
-(fold_plan.h), compiled with g++.
+(fold_plan.h), and of the f-gram index's plan (index_plan.h), compiled with g++.
 
 The plans are plain C++ with no CUDA header, so they run on any host.  Tests use the driver to pin the kernel a call gets
-(test_embed_plan.py, test_fold_plan.py) and to pick, for every kernel the library compiles, a call that launches it
+(test_embed_plan.py, test_fold_plan.py), the shape of an index (test_index_plan.py) and to pick, for every kernel the library compiles, a call that launches it
 (test_gpu_kernel_matrix.py).  A helper module, not a conftest: importing it does nothing until ``PlanDriver`` is built.
 """
 
@@ -17,15 +17,17 @@ from typing import Iterable, List, Optional, Sequence, Tuple
 CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "scone_b200", "csrc")
 FAMILIES = ("bulk", "pipe", "ldg")
 
-# argv: shapes | plan <sms> | detail <sms> | fold <sms>.  plan / detail read one call per line:
+# argv: shapes | plan <sms> | detail <sms> | fold <sms> | index.  plan / detail read one call per line:
 # D row_stride pos additive resolved P SCONE_EMBED_PIPE(or -) T
-# and fold reads: quant H K k SCONE_FOLD_2SM(or -) SCONE_FOLD_XCH(or -) resident_exchange_clusters
+# fold reads: quant H K k SCONE_FOLD_2SM(or -) SCONE_FOLD_XCH(or -) resident_exchange_clusters
+# and index reads: n max_n max_tok load_factor SCONE_INDEX_FORMAT(or -) SCONE_INDEX_FILTER(or -)
 SOURCE = r"""
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include "embed_plan.h"
 #include "fold_plan.h"
+#include "index_plan.h"
 using namespace scone;
 static int fold(int sms) {
     const char *path[kNumFoldPaths] = {"single", "pairs", "pairtile", "exchange"};
@@ -42,6 +44,18 @@ static int fold(int sms) {
     }
     return 0;
 }
+static int index() {
+    long long n;
+    int max_n, max_tok;
+    double lf;
+    char fmt[32], filt[32];
+    while (scanf("%lld %d %d %lf %31s %31s", &n, &max_n, &max_tok, &lf, fmt, filt) == 6) {
+        const IndexPlan pl = plan_index(IndexCall{n, max_n, max_tok, lf, fmt[0] == '-' ? nullptr : fmt, filt[0] == '-' ? nullptr : filt});
+        printf("%s format %d slot_bytes %d cap %llu filter_words %u filter_always %d\n", kSlotFormats[pl.format].name,
+               (int)pl.format, kSlotFormats[pl.format].slot_bytes, (unsigned long long)pl.cap, pl.filter_words, (int)pl.filter_always);
+    }
+    return 0;
+}
 int main(int argc, char **argv) {
     const char *fam[3] = {"bulk", "pipe", "ldg"};
     if (argc == 2 && !strcmp(argv[1], "shapes")) {
@@ -51,6 +65,7 @@ int main(int argc, char **argv) {
         }
         return 0;
     }
+    if (argc == 2 && !strcmp(argv[1], "index")) return index();
     if (argc != 3) return 2;
     if (!strcmp(argv[1], "fold")) return fold(atoi(argv[2]));
     const bool detail = !strcmp(argv[1], "detail");
@@ -83,6 +98,8 @@ int main(int argc, char **argv) {
 Call = Tuple[int, int, int, int, int, int, Optional[str], int]
 # (quant, H, K, k, SCONE_FOLD_2SM or None, SCONE_FOLD_XCH or None, resident exchange clusters)
 FoldCall = Tuple[int, int, int, int, Optional[str], Optional[str], int]
+# (n, max_n, largest token, load factor, SCONE_INDEX_FORMAT or None, SCONE_INDEX_FILTER or None)
+IndexCall = Tuple[int, int, int, float, Optional[str], Optional[str]]
 
 
 class ShapeRow:
@@ -154,3 +171,8 @@ class PlanDriver:
         cases = list(cases)
         return self._lines(["fold", str(sms)], "".join(f"{q} {H} {K} {k} {s or '-'} {x or '-'} {res}\n" for q, H, K, k, s, x, res in cases),
                            len(cases))
+
+    def index(self, cases: Iterable[IndexCall]) -> List[str]:
+        """plan_index() of each call: the slot format's name, number and size, the capacity, the filter words and filter_always."""
+        cases = list(cases)
+        return self._lines(["index"], "".join(f"{n} {m} {t} {lf!r} {f or '-'} {x or '-'}\n" for n, m, t, lf, f, x in cases), len(cases))

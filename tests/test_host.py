@@ -143,7 +143,7 @@ def _device_hash(tokens_reversed: np.ndarray, n: int) -> np.ndarray:
 
 @pytest.mark.parametrize("n_keys", [50_000, 300_000, 1_000_000])
 def test_prefilter_parameters_give_the_documented_false_positive_rate(n_keys):
-    """The index's Bloom pre-filter (common.cuh: filter_bits / filter_pass, index.cu: sizing) restated in numpy: 16+ bits per
+    """The index's Bloom pre-filter (index_format.cuh: filter_bits / filter_pass, index_plan.h: sizing) restated in numpy: 16+ bits per
     f-gram, two bits of one 32-bit word per key -> no false negatives, false positives of a few per cent at most (DESIGN.md
     section 3 quotes ~1.5 %).  Checks the design parameters; the CUDA code itself is held to the oracle by the GPU tests."""
     u = np.uint64
@@ -155,7 +155,7 @@ def test_prefilter_parameters_give_the_documented_false_positive_rate(n_keys):
     words = (words + 31) & ~31
     assert 16 * n_keys <= 32 * words < 16 * n_keys + 32 * 1024 + 1024
     def word_and_bits(h):
-        w = ((h & u(0xFFFFFFFF)) * u(words)) >> u(32)     # common.cuh: filter_word
+        w = ((h & u(0xFFFFFFFF)) * u(words)) >> u(32)     # index_format.cuh: filter_word
         b = (u(1) << ((h >> u(32)) & u(31))) | (u(1) << ((h >> u(37)) & u(31)))
         return w.astype(np.int64), b.astype(np.uint32)
     filt = np.zeros(words, dtype=np.uint32)
@@ -411,7 +411,7 @@ def test_bench_byte_accounting_matches_the_survey_formula():
 
 
 def test_compact20_slot_packing_is_injective():
-    """numpy restatement of common.cuh::pack_key20 (a 28-bit id + five 20-bit tokens, reverse order, 0xFFFFF padded, in 16 bytes):
+    """numpy restatement of index_format.cuh::Compact20Slot::pack (a 28-bit id + five 20-bit tokens, reverse order, 0xFFFFF padded, in 16 bytes):
     the four words determine (length, tokens) uniquely and the id survives next to the four spare token bits; the all-ones word
     that marks an empty slot cannot be produced by a valid entry (ids < 2^28 - 1)."""
     PAD = 0xFFFFF
